@@ -1,13 +1,17 @@
 #!/usr/bin/env python
 """Benchmark of the VTMAE train step (BASELINE.json metric: train samples/sec, fwd+bwd+AdamW).
 
-    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl reference]
+    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl reference] [--dump-outputs DIR]
 
 Workload (BASELINE.json configs[1]): the canonical train.py model (64x64x12 image frame-stack +
 two 32x32x12 tactile maps, dim 256, enc 4x / dec 3x, mask 0.95, early_conv_masking=False),
 batch 256 per GPU, bf16 tensor-core compute with fp32 master weights / accumulation, synthetic
 data, random-init weights.  One "step" = zero_grad + forward + backward (+ gradient all-reduce for
-N > 1) + clip_grad_norm_(0.5) + AdamW, i.e. /root/reference/models/pretrain_models.py:707-711.
+N > 1) + clip_grad_norm_(0.5) + AdamW, i.e. the reference's models/pretrain_models.py:707-711.
+
+`--dump-outputs DIR` writes, after the K timed steps, what the last of them handed back to its caller
+(see dump_outputs) as DIR/<name>.npy.  Weights and inputs are seeded, so the same arguments give the same
+inputs on every run and two builds of the project can be compared output for output.
 
 Prints ONE JSON line on rank 0.  `value` = whole-job samples/s with inputs resident in HBM;
 `e2e` = the same metric through the public module API with pinned HOST inputs (H2D copy of every
@@ -158,7 +162,7 @@ def run_reference_arm(args):
     rank = int(os.environ.get("RANK", "0"))
     if rank != 0:
         return
-    steps = max(1, min(args.steps, 40))
+    steps = args.steps
     sps, ms, cores = cpu_reference_run(steps, max(1, min(args.warmup, 3)))
     sample = f"batch 32 slice of the 256/GPU workload, fp32, torch CPU, {cores} threads, {steps} timed steps"
     line = {"impl": "reference", "metric": "VTMAE train samples/sec (fwd+bwd+AdamW)", "value": sps, "unit": "samples/s",
@@ -320,6 +324,31 @@ def _clocks_record(burst_sampler, sustained):
     return rec
 
 
+DUMP_LIMIT_BYTES = 64 << 20
+
+
+def dump_outputs(out_dir, mae, loss):
+    """What one train step hands back to its caller, as float32 DIR/<name>.npy: `loss`, and for every parameter
+    `param.<name>` (the fp32 master weight after the AdamW update) and `grad.<name>` (its gradient as left in .grad,
+    i.e. after clipping; only parameters the step gives a gradient).  For the benchmark model that is all of it, about
+    41 MB, so nothing is sampled."""
+    import numpy as np
+    arrays = {"loss": loss}
+    for name in mae.arena.names:
+        p = mae.arena.params[name]
+        arrays[f"param.{name}"] = p
+        if p.grad is not None:
+            arrays[f"grad.{name}"] = p.grad
+    arrays = {k: v.detach().float().cpu().numpy() for k, v in arrays.items()}
+    total = sum(a.nbytes for a in arrays.values())
+    if total > DUMP_LIMIT_BYTES:
+        raise SystemExit(f"--dump-outputs: {total} bytes exceed the {DUMP_LIMIT_BYTES} byte limit")
+    out = Path(out_dir)
+    out.mkdir(parents=True, exist_ok=True)
+    for k, a in arrays.items():
+        np.save(out / f"{k}.npy", a)
+
+
 def _teardown(world, trainer=None):
     """Multi-rank exit: the step graphs hold captured NCCL kernels, and tearing the communicator down while they are
     alive (or letting the interpreter do it in arbitrary order at exit) can block for minutes.  Order: all ranks
@@ -394,6 +423,8 @@ def run_gpu_arm(args):
     ms_per_step = ms_total / args.steps
     value = B * world * args.steps / (ms_total * 1e-3)
     loss_val = float(loss.item())
+    if args.dump_outputs and rank == 0:        # replicas are identical: rank 0 speaks for all
+        dump_outputs(args.dump_outputs, mae, loss)
     if args.profile:
         if rank == 0:
             print(json.dumps({"profile_run": True, "ms_per_step": ms_per_step, "value": value, "loss": loss_val}), flush=True)
@@ -711,7 +742,13 @@ def main():
                     help="BASELINE.json workload: 2 = headline (configs[1]); 3 = vision-only, global batch 1024; 4 = DINO-tac-MAE, global batch 512")
     ap.add_argument("--sustain-seconds", type=float, default=3.0,
                     help="also time the device-resident loop for at least this long (0 disables)")
+    ap.add_argument("--dump-outputs", metavar="DIR",
+                    help="write the loss, parameters and gradients of the last timed step as DIR/<name>.npy")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and (args.impl != "m3l_b200" or args.config != 2):
+        ap.error("--dump-outputs is available for the headline workload (--config 2, --impl m3l_b200)")
     if args.impl == "reference":
         run_reference_arm(args)
     elif args.config in (3, 4):

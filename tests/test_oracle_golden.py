@@ -36,8 +36,15 @@ def test_oracle_matches_reference_golden(name):
     grads = {k: (sd[k].grad if present.get(k, True) else None) for k in keys}
     total = O.clip_and_adamw(sd, grads, st)
     assert torch.allclose(total, g.t("grad_total_norm"), rtol=1e-5)
+    # A first AdamW step moves a weight by lr * g / (|g| + eps), g the clipped gradient.  Entries with |g| far below
+    # eps = 1e-8 are rounding noise of a cancelling sum (~1e-10, their value set by the CPU's summation order: thread
+    # count, SIMD width), which that step amplifies by lr / eps.  So the bound adds a gradient error of 1e-9 carried
+    # through the step, lr * eps * 1e-9 / (|g| + eps)^2: ~1e-9 wherever |g| >> eps, lr / 10 where |g| << eps.
+    coef = min(1.0, 0.5 / (float(total) + 1e-6))
     for k, w in g.after().items():
-        assert torch.allclose(sd[k].detach(), w, rtol=1e-6, atol=1e-7), k
+        gr = grads[k]
+        carried = 0.0 if gr is None else 1e-4 * 1e-8 * 1e-9 / (gr.abs() * coef + 1e-8) ** 2
+        assert ((sd[k].detach() - w).abs() <= 1e-7 + 1e-6 * w.abs() + carried).all(), k
     with torch.no_grad():
         loss2 = O.vtmae_forward(sd, cfg, x, noise)
     assert torch.allclose(loss2, g.t("loss_after_step"), rtol=1e-5)
