@@ -275,7 +275,8 @@ int m3l_token_mean_fwd(const void* x_bf16, int batch, int n_tokens, int dim, flo
 int m3l_token_mean_bwd(const float* dout, int batch, int n_tokens, int dim, void* dx_bf16, void* stream);
 
 /* ------------------------------------------------------------------------------------------
- * Fused multi-head attention, sequence length n <= 256, dim_head == 64 (tcgen05 / TMEM / TMA).
+ * Fused multi-head attention, sequence length n <= 256 (longer sequences: m3l_attention_long_* below),
+ * dim_head == 64 (tcgen05 / TMEM / TMA).
  * Replaces vit_pytorch Attention's softmax(q k^T * scale) v and its backward
  * (pretrain_models.py:113,784 through vit-pytorch 1.6.4).
  *   qkv   bf16 [batch*n, 3*heads*64]: columns [q | k | v], head h at h*64 inside each third
@@ -290,6 +291,19 @@ int m3l_attention_fwd(const void* qkv_bf16, int batch, int n, int heads, int dim
 int m3l_attention_bwd(const void* qkv_bf16, const void* out_bf16, const void* dout_bf16,
                       const float* lse, const float* delta, int batch, int n, int heads, int dim_head,
                       float scale, void* dqkv_bf16, void* stream);
+
+/* ------------------------------------------------------------------------------------------
+ * The same two operations for any sequence length n >= 1 (dim_head == 64, else status 3), with the
+ * same arguments, layouts and LSE: FlashAttention-style kernels over 128-key tiles with an online
+ * softmax (attention_long.cu).  m3l_attention_fwd/bwd cover n <= 256; longer sequences go through
+ * these.  The backward is two kernels (dK / dV key-tile-stationary, dQ query-tile-stationary),
+ * deterministic (no atomics), and allocates nothing.
+ * ---------------------------------------------------------------------------------------- */
+int m3l_attention_long_fwd(const void* qkv_bf16, int batch, int n, int heads, int dim_head, float scale,
+                           void* out_bf16, float* lse, void* stream);
+int m3l_attention_long_bwd(const void* qkv_bf16, const void* out_bf16, const void* dout_bf16,
+                           const float* lse, const float* delta, int batch, int n, int heads, int dim_head,
+                           float scale, void* dqkv_bf16, void* stream);
 
 /* ------------------------------------------------------------------------------------------
  * Optimizer over flat fp32 arenas: clip_grad_norm_(params, max_norm) + AdamW.step()

@@ -211,7 +211,7 @@ class DinoV2(nn.Module):
         for blk in prep["blocks"]:
             y, _ = ops.layernorm_fwd(xs, *blk["n1"], eps=1e-6, want_stats=False)
             qkv = ops.gemm(y, blk["wqkv"], bias=blk["bqkv"])
-            o, _ = ops.attention_fwd(qkv, B, n, heads, 64, scale)
+            o, _ = ops.mha_fwd(qkv, B, n, heads, 64, scale)
             xs = ops.gemm(o, blk["wproj"], bias=blk["bproj"], residual=xs)
             y, _ = ops.layernorm_fwd(xs, *blk["n2"], eps=1e-6, want_stats=False)
             h = ops.gemm(y, blk["w1"], bias=blk["b1"], act=ops.GELU_FWD)

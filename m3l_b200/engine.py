@@ -197,7 +197,7 @@ def stack_fwd(A: ParamArena, spec: StackSpec, x: torch.Tensor, B: int, n: int, s
         xn1, st1 = ops.layernorm_fwd(x, A.f32(pa + ".norm.weight"), A.f32(pa + ".norm.bias"),
                                      want_stats=saved is not None)
         qkv = ops.gemm(xn1, A.bf(pa + ".to_qkv.weight"))
-        o, lse = ops.attention_fwd(qkv, B, n, spec.heads, spec.dim_head, scale)
+        o, lse = ops.mha_fwd(qkv, B, n, spec.heads, spec.dim_head, scale)
         fused = _FUSED_MLP and ops.ln_mlp_supported(spec.dim, spec.mlp_dim)
         # training keeps x_mid for the backward pass, so the attention-output GEMM writes its result twice (x_mid and
         # the buffer the fused feed-forward block then accumulates into); inference updates x_mid in place
@@ -253,7 +253,7 @@ def stack_bwd(A: ParamArena, G: GradView, spec: StackSpec, dx: torch.Tensor, B: 
         # dO, and in the same epilogue delta = rowsum(dO * O) per head (dim_head == 64 == one epilogue round)
         delta = torch.empty((M, spec.heads), dtype=torch.float32, device=dx.device) if spec.dim_head == 64 else None
         do = ops.gemm(dx_mid, A.bf_t(pa + ".to_out.0.weight"), dot_side=o if delta is not None else None, dot_out=delta)
-        dqkv = ops.attention_bwd(qkv, o, do, lse, B, n, spec.heads, spec.dim_head, scale, delta=delta)
+        dqkv = ops.mha_bwd(qkv, o, do, lse, B, n, spec.heads, spec.dim_head, scale, delta=delta)
         fork.wgrad(dqkv, xn1, G(pa + ".to_qkv.weight"))
         prev_bias = G(f"{spec.prefix}.layers.{l - 1}.1.net.4.bias") if l > 0 else None
         dx_in = _dgrad_ln_bwd(dqkv, A.bf_t(pa + ".to_qkv.weight"), x, st1, A.f32(pa + ".norm.weight"),

@@ -431,6 +431,50 @@ def attention_bwd(qkv, out, dout, lse, batch, n, heads, dim_head, scale, *, dqkv
     return dqkv
 
 
+def attention_long_fwd(qkv, batch, n, heads, dim_head, scale, *, out=None, lse=None):
+    """attention_fwd for any n >= 1 (csrc/attention_long.cu: 128-key tiles, online softmax); same outputs."""
+    _req_cuda(qkv)
+    inner = heads * dim_head
+    assert qkv.dtype == torch.bfloat16 and qkv.is_contiguous() and qkv.shape == (batch * n, 3 * inner)
+    if out is None:
+        out = torch.empty((batch * n, inner), dtype=torch.bfloat16, device=qkv.device)
+    if lse is None:
+        lse = torch.empty((batch, heads, n), dtype=torch.float32, device=qkv.device)
+    check(_lib.load().m3l_attention_long_fwd(ptr(qkv), batch, n, heads, dim_head, C.c_float(scale), ptr(out), ptr(lse),
+                                             current_stream()), "m3l_attention_long_fwd")
+    return out, lse
+
+
+def attention_long_bwd(qkv, out, dout, lse, batch, n, heads, dim_head, scale, *, dqkv=None, delta=None):
+    """attention_bwd for any n >= 1 (two deterministic kernels: dK / dV per key tile, dQ per query tile)."""
+    _req_cuda(qkv, out, dout, lse, dqkv, delta)
+    if dqkv is None:
+        dqkv = torch.empty_like(qkv)
+    assert dout.is_contiguous() and out.is_contiguous()
+    assert delta is None or (delta.dtype == torch.float32 and delta.is_contiguous() and delta.shape == (batch * n, heads))
+    check(_lib.load().m3l_attention_long_bwd(ptr(qkv), ptr(out), ptr(dout), ptr(lse), ptr(delta), batch, n, heads,
+                                             dim_head, C.c_float(scale), ptr(dqkv), current_stream()),
+          "m3l_attention_long_bwd")
+    return dqkv
+
+
+# longest sequence the single-CTA kernels of csrc/attention.cu take; above it csrc/attention_long.cu runs
+SHORT_ATTENTION_MAX_N = 256
+
+
+def mha_fwd(qkv, batch, n, heads, dim_head, scale, *, out=None, lse=None):
+    """Multi-head attention forward for any sequence length: attention_fwd up to SHORT_ATTENTION_MAX_N tokens,
+    attention_long_fwd above.  The one place the model code picks between the two kernel families."""
+    f = attention_fwd if n <= SHORT_ATTENTION_MAX_N else attention_long_fwd
+    return f(qkv, batch, n, heads, dim_head, scale, out=out, lse=lse)
+
+
+def mha_bwd(qkv, out, dout, lse, batch, n, heads, dim_head, scale, *, dqkv=None, delta=None):
+    """Backward of mha_fwd (same selection by n)."""
+    f = attention_bwd if n <= SHORT_ATTENTION_MAX_N else attention_long_bwd
+    return f(qkv, out, dout, lse, batch, n, heads, dim_head, scale, dqkv=dqkv, delta=delta)
+
+
 # ------------------------------------------------------------------------------------------
 # optimizer
 # ------------------------------------------------------------------------------------------
