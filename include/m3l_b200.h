@@ -306,6 +306,18 @@ int m3l_attention_long_bwd(const void* qkv_bf16, const void* out_bf16, const voi
                            float scale, void* dqkv_bf16, void* stream);
 
 /* ------------------------------------------------------------------------------------------
+ * The same two operations for 32- and 128-wide heads (dim_head 32 or 128, else status 3; 64-wide
+ * heads use the entry points above), any n >= 1, with the same arguments, layouts, LSE and
+ * deterministic two-kernel backward as m3l_attention_long_*: the other instantiations of the same
+ * kernels (attention_long.cuh, attention_dh.cu).  `delta` is optional as above.
+ * ---------------------------------------------------------------------------------------- */
+int m3l_attention_dh_fwd(const void* qkv_bf16, int batch, int n, int heads, int dim_head, float scale,
+                         void* out_bf16, float* lse, void* stream);
+int m3l_attention_dh_bwd(const void* qkv_bf16, const void* out_bf16, const void* dout_bf16,
+                         const float* lse, const float* delta, int batch, int n, int heads, int dim_head,
+                         float scale, void* dqkv_bf16, void* stream);
+
+/* ------------------------------------------------------------------------------------------
  * Optimizer over flat fp32 arenas: clip_grad_norm_(params, max_norm) + AdamW.step()
  * (pretrain_models.py:670-676,707-711; torch.optim.AdamW defaults).  `state` is 8 doubles on the
  * device: [0] step counter, [1] sum of squares of all gradients (zero it, then call

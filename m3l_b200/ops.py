@@ -458,20 +458,58 @@ def attention_long_bwd(qkv, out, dout, lse, batch, n, heads, dim_head, scale, *,
     return dqkv
 
 
+def attention_dh_fwd(qkv, batch, n, heads, dim_head, scale, *, out=None, lse=None):
+    """attention_long_fwd for 32- and 128-wide heads (csrc/attention_dh.cu), any n >= 1; same outputs."""
+    _req_cuda(qkv)
+    inner = heads * dim_head
+    assert qkv.dtype == torch.bfloat16 and qkv.is_contiguous() and qkv.shape == (batch * n, 3 * inner)
+    if out is None:
+        out = torch.empty((batch * n, inner), dtype=torch.bfloat16, device=qkv.device)
+    if lse is None:
+        lse = torch.empty((batch, heads, n), dtype=torch.float32, device=qkv.device)
+    check(_lib.load().m3l_attention_dh_fwd(ptr(qkv), batch, n, heads, dim_head, C.c_float(scale), ptr(out), ptr(lse),
+                                           current_stream()), "m3l_attention_dh_fwd")
+    return out, lse
+
+
+def attention_dh_bwd(qkv, out, dout, lse, batch, n, heads, dim_head, scale, *, dqkv=None, delta=None):
+    """attention_long_bwd for 32- and 128-wide heads (the same two deterministic kernels)."""
+    _req_cuda(qkv, out, dout, lse, dqkv, delta)
+    if dqkv is None:
+        dqkv = torch.empty_like(qkv)
+    assert dout.is_contiguous() and out.is_contiguous()
+    assert delta is None or (delta.dtype == torch.float32 and delta.is_contiguous() and delta.shape == (batch * n, heads))
+    check(_lib.load().m3l_attention_dh_bwd(ptr(qkv), ptr(out), ptr(dout), ptr(lse), ptr(delta), batch, n, heads,
+                                           dim_head, C.c_float(scale), ptr(dqkv), current_stream()),
+          "m3l_attention_dh_bwd")
+    return dqkv
+
+
 # longest sequence the single-CTA kernels of csrc/attention.cu take; above it csrc/attention_long.cu runs
 SHORT_ATTENTION_MAX_N = 256
+# head widths with kernels: 64 (attention.cu / attention_long.cu), 32 and 128 (attention_dh.cu)
+ATTENTION_HEAD_DIMS = (32, 64, 128)
+
+
+def _mha_kernels(n, dim_head):
+    if dim_head != 64:
+        return attention_dh_fwd, attention_dh_bwd
+    if n <= SHORT_ATTENTION_MAX_N:
+        return attention_fwd, attention_bwd
+    return attention_long_fwd, attention_long_bwd
 
 
 def mha_fwd(qkv, batch, n, heads, dim_head, scale, *, out=None, lse=None):
-    """Multi-head attention forward for any sequence length: attention_fwd up to SHORT_ATTENTION_MAX_N tokens,
-    attention_long_fwd above.  The one place the model code picks between the two kernel families."""
-    f = attention_fwd if n <= SHORT_ATTENTION_MAX_N else attention_long_fwd
+    """Multi-head attention forward for any sequence length.  64-wide heads: attention_fwd up to
+    SHORT_ATTENTION_MAX_N tokens, attention_long_fwd above; 32- and 128-wide heads: attention_dh_fwd for every n.
+    The one place the model code picks between the kernel families."""
+    f = _mha_kernels(n, dim_head)[0]
     return f(qkv, batch, n, heads, dim_head, scale, out=out, lse=lse)
 
 
 def mha_bwd(qkv, out, dout, lse, batch, n, heads, dim_head, scale, *, dqkv=None, delta=None):
-    """Backward of mha_fwd (same selection by n)."""
-    f = attention_bwd if n <= SHORT_ATTENTION_MAX_N else attention_long_bwd
+    """Backward of mha_fwd (same selection by n and dim_head)."""
+    f = _mha_kernels(n, dim_head)[1]
     return f(qkv, out, dout, lse, batch, n, heads, dim_head, scale, dqkv=dqkv, delta=delta)
 
 

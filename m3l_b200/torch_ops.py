@@ -16,6 +16,7 @@ What each op stands in for in the reference (paths under /root/reference):
   m3l::layernorm_fwd / layernorm_bwd      nn.LayerNorm (vit_pytorch blocks, patch embedding, final norms)
   m3l::attention_fwd / attention_bwd      softmax(q k^T / sqrt(d)) v of vit_pytorch.Attention, fused (n <= 256)
   m3l::attention_long_fwd / attention_long_bwd   the same for any sequence length (online softmax over key tiles)
+  m3l::attention_dh_fwd / attention_dh_bwd       the same for 32- and 128-wide heads, any sequence length
   m3l::ln_mlp_fwd / ln_mlp_bwd            x + FeedForward(x) of vit_pytorch.Transformer as one kernel each way
   m3l::mask_indices   torch.rand(...).argsort() split into masked / unmasked (models/pretrain_models.py:229-248)
   m3l::patch_layernorm                    Rearrange('b c (h p1) (w p2) -> b (h w) (p1 p2 c)') + gather + LayerNorm (:164-198,766-779)
@@ -158,6 +159,24 @@ def _attn_long_bwd(qkv: Tensor, out: Tensor, dout: Tensor, lse: Tensor, batch: i
 
 _define("attention_long_bwd(Tensor qkv, Tensor out, Tensor dout, Tensor lse, int batch, int n, int heads, int dim_head, "
         "float scale) -> Tensor", _attn_long_bwd, _attn_bwd_fake)
+
+
+def _attn_dh_fwd(qkv: Tensor, batch: int, n: int, heads: int, dim_head: int, scale: float) -> Tuple[Tensor, Tensor]:
+    return ops.attention_dh_fwd(qkv.contiguous(), batch, n, heads, dim_head, scale)
+
+
+_define("attention_dh_fwd(Tensor qkv, int batch, int n, int heads, int dim_head, float scale) -> (Tensor, Tensor)",
+        _attn_dh_fwd, _attn_fwd_fake)
+
+
+def _attn_dh_bwd(qkv: Tensor, out: Tensor, dout: Tensor, lse: Tensor, batch: int, n: int, heads: int, dim_head: int,
+                 scale: float) -> Tensor:
+    return ops.attention_dh_bwd(qkv.contiguous(), out.contiguous(), dout.contiguous(), lse.contiguous(), batch, n, heads,
+                                dim_head, scale)
+
+
+_define("attention_dh_bwd(Tensor qkv, Tensor out, Tensor dout, Tensor lse, int batch, int n, int heads, int dim_head, "
+        "float scale) -> Tensor", _attn_dh_bwd, _attn_bwd_fake)
 
 
 # ---------------------------------------------------------------------------------------------- fused feed-forward block

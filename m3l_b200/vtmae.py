@@ -61,8 +61,9 @@ class Transformer(nn.Module):
 
     def __init__(self, dim, depth, heads, dim_head, mlp_dim, dropout=0.0):
         super().__init__()
-        if dim_head != 64:
-            raise M3LError(f"dim_head={dim_head}: the sm_100a attention kernel supports dim_head == 64 only")
+        if dim_head not in ops.ATTENTION_HEAD_DIMS:
+            raise M3LError(f"dim_head={dim_head}: the sm_100a attention kernels support dim_head in "
+                           f"{ops.ATTENTION_HEAD_DIMS} only")
         self.dim, self.depth, self.heads, self.dim_head, self.mlp_dim, self.p_drop = dim, depth, heads, dim_head, mlp_dim, dropout
         self.norm = nn.LayerNorm(dim)
         self.layers = nn.ModuleList([])
