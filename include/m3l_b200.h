@@ -71,6 +71,15 @@ typedef struct m3l_gemm_args {
   float* ln_dgamma;       /* fp32 [256], accumulated */
   float* ln_dbeta;        /* fp32 [256], accumulated */
   float* ln_dxcol;        /* fp32 [256] or NULL, accumulated */
+  /* Dropout (drop_key != NULL; training mode of vit_pytorch's FeedForward / Attention.to_out Dropout layers).  The
+   * mask Z is m3l_b200's counter-based one (see m3l_dropout_bwd), with row / column of the output, plane 0 and site
+   * drop_site; Z is 0 or 65536 / (65536 - thr), thr = floor(drop_p * 65536 + 0.5).  Two epilogues take it:
+   *   act 1 (GELU), no residual:   out = Z o GELU(acc + bias), aux_out = Z o GELU'(acc + bias)
+   *   act 0 with a residual:       out = residual + Z o (acc + bias) (and out2 the same)
+   * Any other combination, drop_p outside [0, 1), and drop_p > 0 with a NULL key return status 1. */
+  const int64_t* drop_key;  /* device int64 [1]: the 64-bit Philox key, or NULL */
+  int32_t drop_site;        /* (layer << 2) | site */
+  float drop_p;
 } m3l_gemm_args;
 
 int m3l_gemm_bf16(const m3l_gemm_args* args, void* stream);
@@ -316,6 +325,34 @@ int m3l_attention_dh_fwd(const void* qkv_bf16, int batch, int n, int heads, int 
 int m3l_attention_dh_bwd(const void* qkv_bf16, const void* out_bf16, const void* dout_bf16,
                          const float* lse, const float* delta, int batch, int n, int heads, int dim_head,
                          float scale, void* dqkv_bf16, void* stream);
+
+/* ------------------------------------------------------------------------------------------
+ * Dropout (training mode of vit_pytorch's Attention / FeedForward Dropout layers).
+ *
+ * The mask is a pure function of logical coordinates: Philox4x32-10 (Random123) under the 64-bit key *drop_key
+ * (device memory), counter (col >> 3, row, plane, site); the four output words are eight 16-bit uniforms, low half
+ * first, and element `col & 7` is kept iff its uniform u >= thr = floor(p * 65536 + 0.5).  Kept elements are
+ * multiplied by 65536 / (65536 - thr) (fp32).  site = (layer << 2) | s with s = 0 attention probabilities,
+ * 1 attention output (to_out), 2 after the feed-forward GELU, 3 feed-forward output.  Every entry point returns
+ * status 1 for p outside [0, 1) or NaN and for a NULL key with p > 0.
+ *
+ * m3l_attention_dropout_fwd/bwd: m3l_attention_long_fwd/bwd with dropout on the attention probabilities
+ * (row = query index, col = key index, plane = sample * heads + head), dim_head 32, 64 or 128 (else status 3), any
+ * n.  The forward's lse is that of the undropped scores; out = (P o Z) V.  The backward takes the same optional
+ * delta = rowsum(dout * out).  At p = 0 the results equal the kernels without dropout bit for bit.
+ *
+ * m3l_dropout_bwd: out = Z o dy for a contiguous bf16 [rows, cols] matrix (plane 0), and colsum[c] += sum_r out[r, c]
+ * (fp32) when colsum is not NULL.  It is the backward of a dropout applied by m3l_gemm_bf16's dropout epilogues.
+ * ---------------------------------------------------------------------------------------- */
+int m3l_attention_dropout_fwd(const void* qkv_bf16, int batch, int n, int heads, int dim_head, float scale,
+                              const int64_t* drop_key, int drop_site, float drop_p, void* out_bf16, float* lse,
+                              void* stream);
+int m3l_attention_dropout_bwd(const void* qkv_bf16, const void* out_bf16, const void* dout_bf16,
+                              const float* lse, const float* delta, int batch, int n, int heads, int dim_head,
+                              float scale, const int64_t* drop_key, int drop_site, float drop_p, void* dqkv_bf16,
+                              void* stream);
+int m3l_dropout_bwd(const void* dy_bf16, int rows, int cols, const int64_t* drop_key, int drop_site, float drop_p,
+                    void* out_bf16, float* colsum, void* stream);
 
 /* ------------------------------------------------------------------------------------------
  * Optimizer over flat fp32 arenas: clip_grad_norm_(params, max_norm) + AdamW.step()

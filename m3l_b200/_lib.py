@@ -31,6 +31,7 @@ class GemmArgs(C.Structure):
         ("out2", C.c_void_p), ("dot_side", C.c_void_p), ("ld_dot", C.c_int32), ("dot_out", C.c_void_p),
         ("ln_x", C.c_void_p), ("ln_stats", C.c_void_p), ("ln_gamma", C.c_void_p), ("ln_skip", C.c_void_p),
         ("ln_dgamma", C.c_void_p), ("ln_dbeta", C.c_void_p), ("ln_dxcol", C.c_void_p),
+        ("drop_key", C.c_void_p), ("drop_site", C.c_int32), ("drop_p", C.c_float),
     ]
 
 
@@ -115,7 +116,8 @@ EXPORTED_SYMBOLS = (
     "m3l_layernorm_bwd", "m3l_decoder_assemble_fwd", "m3l_decoder_assemble_bwd", "m3l_rowclass_sum",
     "m3l_mse_loss", "m3l_colsum", "m3l_ln_param_grad", "m3l_attention_fwd", "m3l_attention_bwd",
     "m3l_attention_long_fwd", "m3l_attention_long_bwd",
-    "m3l_attention_dh_fwd", "m3l_attention_dh_bwd", "m3l_grad_sumsq", "m3l_optimizer_step_begin", "m3l_clip_adamw", "m3l_cast_bf16",
+    "m3l_attention_dh_fwd", "m3l_attention_dh_bwd", "m3l_attention_dropout_fwd", "m3l_attention_dropout_bwd",
+    "m3l_dropout_bwd", "m3l_grad_sumsq", "m3l_optimizer_step_begin", "m3l_clip_adamw", "m3l_cast_bf16",
     "m3l_transpose_cast_bf16", "m3l_token_mean_fwd", "m3l_token_mean_bwd",
     "m3l_im2col", "m3l_col2im_relu", "m3l_token_finish", "m3l_token_finish_bwd", "m3l_vt_load", "m3l_patchify", "m3l_row_scatter_add", "m3l_ema_update",
 )

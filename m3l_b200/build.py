@@ -29,7 +29,8 @@ NVCC_FLAGS = [
 # --use_fast_math only where the approximate exp2 / reciprocal are the point (softmax exponentials and the GELU
 # epilogues of the tensor-core kernels).  LayerNorm statistics, the MSE loss, the gradient norm and AdamW
 # (elementwise.cu, optim.cu) are compiled with IEEE division / sqrt and without flush-to-zero.
-FAST_MATH_SOURCES = {"gemm.cu", "gemm_gelu.cu", "attention.cu", "attention_long.cu", "attention_dh.cu", "rowblock.cu"}
+FAST_MATH_SOURCES = {"gemm.cu", "gemm_gelu.cu", "attention.cu", "attention_long.cu", "attention_dh.cu",
+                     "attention_dropout.cu", "rowblock.cu"}
 
 
 def flags_for(src: Path) -> list[str]:

@@ -43,6 +43,7 @@
 //                  dh = 128).
 #pragma once
 #include "common.cuh"
+#include "dropout.cuh"
 #include "m3l_internal.h"
 
 namespace m3l {
@@ -170,9 +171,11 @@ struct LongFwdParams {
   float scale;
 };
 
-template <int kDh>
-__global__ void __launch_bounds__(192, 1)
-attn_long_fwd_kernel(const __grid_constant__ CUtensorMap map_qkv, const LongFwdParams p) {
+// kDrop: dropout on the probabilities that multiply V (attention_dropout.cu).  The row sums and the LSE use the
+// undropped P, so lse equals the lse without dropout.
+template <int kDh, bool kDrop>
+__device__ __forceinline__ void attn_long_fwd_body(const CUtensorMap& map_qkv, const LongFwdParams& p,
+                                                   const DropParams& dp) {
   using Cfg = LongCfg<kDh>;
   constexpr int kTileBytes = Cfg::kTileBytes, kFwdStages = Cfg::kFwdStages, kN = Cfg::kN;
   extern __shared__ uint8_t smem_raw[];
@@ -290,6 +293,8 @@ attn_long_fwd_kernel(const __grid_constant__ CUtensorMap map_qkv, const LongFwdP
     const uint32_t p_u32 = smem_u32(sP);
     const float sl2 = p.scale * kLog2e;
     const f32x2 sl2_2 = f2_splat(sl2);
+    uint64_t dkey = 0;
+    if constexpr (kDrop) dkey = drop_key_load(dp.key);
     int g = 0;
     for (int item = blockIdx.x; item < p.num_items; item += gridDim.x) {
       const int t = item % p.tiles, bh = item / p.tiles;
@@ -300,6 +305,11 @@ attn_long_fwd_kernel(const __grid_constant__ CUtensorMap map_qkv, const LongFwdP
         const int slot = g & 1;
         const int kvalid = min(kTile, n - j * kTile);   // keys of this tile inside the sequence (>= 1)
         const uint32_t ts = t_lane + slot * kTile;
+        uint32_t keep[4];                               // kDrop: keep bits of the tile's 128 keys, while S is computed
+        if constexpr (kDrop) {
+#pragma unroll
+          for (int q = 0; q < 4; ++q) keep[q] = drop_keep32(dkey, j * kTile + q * 32, t * kTile + row, bh, dp.site, dp.thr);
+        }
         mbar_wait(&bars->s_full[slot], (g >> 1) & 1);
         tc_fence_after_sync();
         // ---- pass 1: tile max, four independent chains
@@ -358,6 +368,10 @@ attn_long_fwd_kernel(const __grid_constant__ CUtensorMap map_qkv, const LongFwdP
                   p1 = col0 + e + 1 < kvalid ? p1 : 0.f;
                 }
                 if (e & 2) sum1 += p0 + p1; else sum0 += p0 + p1;
+                if constexpr (kDrop) {
+                  p0 = (keep[(c + h2)] >> e) & 1u ? p0 * dp.scale : 0.f;
+                  p1 = (keep[(c + h2)] >> (e + 1)) & 1u ? p1 * dp.scale : 0.f;
+                }
                 pw[(col0 + e) >> 1] = pack_bf16x2(p0, p1);
               }
             }
@@ -426,6 +440,18 @@ attn_long_fwd_kernel(const __grid_constant__ CUtensorMap map_qkv, const LongFwdP
   }
 }
 
+template <int kDh>
+__global__ void __launch_bounds__(192, 1)
+attn_long_fwd_kernel(const __grid_constant__ CUtensorMap map_qkv, const LongFwdParams p) {
+  attn_long_fwd_body<kDh, false>(map_qkv, p, DropParams{});
+}
+
+template <int kDh>
+__global__ void __launch_bounds__(192, 1)
+attn_long_drop_fwd_kernel(const __grid_constant__ CUtensorMap map_qkv, const LongFwdParams p, const DropParams dp) {
+  attn_long_fwd_body<kDh, true>(map_qkv, p, dp);
+}
+
 // ------------------------------------------------------------------------------------------
 // backward.  kKV = true: KV-stationary (dK, dV); false: Q-stationary (dQ).
 // TMEM columns: [0,128) S  [128,256) dP  [256,256+kN) dV | dQ  [256+kN,256+2kN) dK
@@ -462,10 +488,11 @@ M3L_DEVINL float row_delta(const bf16* po, const bf16* pd) {
   return acc0 + acc1;
 }
 
-template <int kDh, bool kKV>
-__global__ void __launch_bounds__(320, 1)
-attn_long_bwd_kernel(const __grid_constant__ CUtensorMap map_qkv, const __grid_constant__ CUtensorMap map_do,
-                     const LongBwdParams p) {
+// kDrop: with the dropout mask Z (scale folded in) the P slab is P o Z and dS = P o (Z o dP - delta) scale; delta =
+// rowsum(dO o O) is the same expression as without dropout.
+template <int kDh, bool kKV, bool kDrop>
+__device__ __forceinline__ void attn_long_bwd_body(const CUtensorMap& map_qkv, const CUtensorMap& map_do,
+                                                   const LongBwdParams& p, const DropParams& dp) {
   using Cfg = LongCfg<kDh>;
   constexpr int kTileBytes = Cfg::kTileBytes, kN = Cfg::kN;
   constexpr int kBwdStages = Cfg::bwd_stages(kKV);
@@ -623,6 +650,9 @@ attn_long_bwd_kernel(const __grid_constant__ CUtensorMap map_qkv, const __grid_c
     };
     float lg = 0.f, dl = 0.f;
     if (!kKV) stats(tile * kTile + row, lg, dl);
+    uint64_t dkey = 0;
+    if constexpr (kDrop) dkey = drop_key_load(dp.key);
+    const uint32_t plane = (uint32_t)b * p.heads + h;
     for (int s = 0; s < steps; ++s) {
       const int qi = kKV ? s : tile, kj = kKV ? tile : s;
       const int grow = qi * kTile + row;
@@ -630,6 +660,11 @@ attn_long_bwd_kernel(const __grid_constant__ CUtensorMap map_qkv, const __grid_c
       if (kKV) stats(grow, lg, dl);
       const int key0 = kj * kTile + wg * 64;
       const bool interior = (qi * kTile + quad * 32 + 32 <= n) && (key0 + 64 <= n);   // warp-uniform
+      uint32_t keep[2];                                 // kDrop: keep bits of this thread's 64 keys, while S / dP are computed
+      if constexpr (kDrop) {
+        keep[0] = drop_keep32(dkey, key0, grow, plane, dp.site, dp.thr);
+        keep[1] = drop_keep32(dkey, key0 + 32, grow, plane, dp.site, dp.thr);
+      }
       mbar_wait(&bars->sdp_full, s & 1);
       tc_fence_after_sync();
       uint32_t pw[32], dw[32];
@@ -650,10 +685,18 @@ attn_long_bwd_kernel(const __grid_constant__ CUtensorMap map_qkv, const __grid_c
             float t0, t1;
             f2_unpack(f2_fma(f2_packu(sv[e], sv[e + 1]), sl2_2, nlg2), t0, t1);
             const float p0 = exp2f(t0), p1 = exp2f(t1);
-            const f32x2 ds = f2_mul(f2_mul(f2_pack(p0, p1), f2_add(f2_packu(dv[e], dv[e + 1]), ndl2)), sc2);
+            f32x2 dpv = f2_packu(dv[e], dv[e + 1]);
+            float z0 = 1.f, z1 = 1.f;
+            if constexpr (kDrop) {
+              z0 = (keep[c] >> e) & 1u ? dp.scale : 0.f;
+              z1 = (keep[c] >> (e + 1)) & 1u ? dp.scale : 0.f;
+              dpv = f2_mul(dpv, f2_pack(z0, z1));
+            }
+            const f32x2 ds = f2_mul(f2_mul(f2_pack(p0, p1), f2_add(dpv, ndl2)), sc2);
             float d0, d1;
             f2_unpack(ds, d0, d1);
-            pw[c * 16 + (e >> 1)] = pack_bf16x2(p0, p1);
+            if constexpr (kDrop) pw[c * 16 + (e >> 1)] = pack_bf16x2(p0 * z0, p1 * z1);
+            else pw[c * 16 + (e >> 1)] = pack_bf16x2(p0, p1);
             dw[c * 16 + (e >> 1)] = pack_bf16x2(d0, d1);
           }
         } else {
@@ -663,9 +706,16 @@ attn_long_bwd_kernel(const __grid_constant__ CUtensorMap map_qkv, const __grid_c
             const float p0 = exp2f(fmaf(__uint_as_float(sv[e]), sl2, -lg));
             const float p1 = exp2f(fmaf(__uint_as_float(sv[e + 1]), sl2, -lg));
             const float q0 = (valid && key < n) ? p0 : 0.f, q1 = (valid && key + 1 < n) ? p1 : 0.f;
-            pw[c * 16 + (e >> 1)] = pack_bf16x2(q0, q1);
-            dw[c * 16 + (e >> 1)] = pack_bf16x2(q0 * (__uint_as_float(dv[e]) - dl) * p.scale,
-                                                q1 * (__uint_as_float(dv[e + 1]) - dl) * p.scale);
+            float dp0 = __uint_as_float(dv[e]), dp1 = __uint_as_float(dv[e + 1]);
+            if constexpr (kDrop) {
+              const float z0 = (keep[c] >> e) & 1u ? dp.scale : 0.f, z1 = (keep[c] >> (e + 1)) & 1u ? dp.scale : 0.f;
+              dp0 *= z0;
+              dp1 *= z1;
+              pw[c * 16 + (e >> 1)] = pack_bf16x2(q0 * z0, q1 * z1);
+            } else {
+              pw[c * 16 + (e >> 1)] = pack_bf16x2(q0, q1);
+            }
+            dw[c * 16 + (e >> 1)] = pack_bf16x2(q0 * (dp0 - dl) * p.scale, q1 * (dp1 - dl) * p.scale);
           }
         }
       }
@@ -738,12 +788,27 @@ attn_long_bwd_kernel(const __grid_constant__ CUtensorMap map_qkv, const __grid_c
   }
 }
 
+template <int kDh, bool kKV>
+__global__ void __launch_bounds__(320, 1)
+attn_long_bwd_kernel(const __grid_constant__ CUtensorMap map_qkv, const __grid_constant__ CUtensorMap map_do,
+                     const LongBwdParams p) {
+  attn_long_bwd_body<kDh, kKV, false>(map_qkv, map_do, p, DropParams{});
+}
+
+template <int kDh, bool kKV>
+__global__ void __launch_bounds__(320, 1)
+attn_long_drop_bwd_kernel(const __grid_constant__ CUtensorMap map_qkv, const __grid_constant__ CUtensorMap map_do,
+                          const LongBwdParams p, const DropParams dp) {
+  attn_long_bwd_body<kDh, kKV, true>(map_qkv, map_do, p, dp);
+}
+
 // ------------------------------------------------------------------------------------------
 // host launchers (arguments already checked by the entry points)
 // ------------------------------------------------------------------------------------------
-template <int kDh>
+// kDrop: the dropout kernels (attention_dropout.cu), with the mask of `dp`
+template <int kDh, bool kDrop = false>
 int long_fwd_launch(const char* who, const void* qkv_bf16, int batch, int n, int heads, float scale, void* out_bf16,
-                    float* lse, void* stream) {
+                    float* lse, void* stream, const DropParams& dp = DropParams{}) {
   using Cfg = LongCfg<kDh>;
   const int inner = heads * kDh;
   CUtensorMap map_qkv;
@@ -756,22 +821,32 @@ int long_fwd_launch(const char* who, const void* qkv_bf16, int batch, int n, int
   M3L_REQUIRE(items < (1ll << 31), "%s: too many (sample, head, tile) items", who);
   p.num_items = (int)items;
   static bool configured = false;
-  if (!configured) {
-    M3L_CUDA(cudaFuncSetAttribute(attn_long_fwd_kernel<kDh>, cudaFuncAttributeMaxDynamicSharedMemorySize,
-                                  Cfg::kFwdSmem));
-    configured = true;
-  }
   const int grid = std::min(p.num_items, device_sm_count());
-  M3L_CUDA(launch_kernel(attn_long_fwd_kernel<kDh>, dim3(grid), dim3(192), Cfg::kFwdSmem, (cudaStream_t)stream,
-                         map_qkv, p));
+  if constexpr (kDrop) {
+    if (!configured) {
+      M3L_CUDA(cudaFuncSetAttribute(attn_long_drop_fwd_kernel<kDh>, cudaFuncAttributeMaxDynamicSharedMemorySize,
+                                    Cfg::kFwdSmem));
+      configured = true;
+    }
+    M3L_CUDA(launch_kernel(attn_long_drop_fwd_kernel<kDh>, dim3(grid), dim3(192), Cfg::kFwdSmem, (cudaStream_t)stream,
+                           map_qkv, p, dp));
+  } else {
+    if (!configured) {
+      M3L_CUDA(cudaFuncSetAttribute(attn_long_fwd_kernel<kDh>, cudaFuncAttributeMaxDynamicSharedMemorySize,
+                                    Cfg::kFwdSmem));
+      configured = true;
+    }
+    M3L_CUDA(launch_kernel(attn_long_fwd_kernel<kDh>, dim3(grid), dim3(192), Cfg::kFwdSmem, (cudaStream_t)stream,
+                           map_qkv, p));
+  }
   M3L_CUDA(cudaGetLastError());
   return M3L_OK;
 }
 
-template <int kDh>
+template <int kDh, bool kDrop = false>
 int long_bwd_launch(const char* who, const void* qkv_bf16, const void* out_bf16, const void* dout_bf16,
                     const float* lse, const float* delta, int batch, int n, int heads, float scale, void* dqkv_bf16,
-                    void* stream) {
+                    void* stream, const DropParams& dp = DropParams{}) {
   using Cfg = LongCfg<kDh>;
   M3L_REQUIRE(batch <= 65535, "%s: batch %d > 65535", who, batch);
   const int inner = heads * kDh;
@@ -787,17 +862,32 @@ int long_bwd_launch(const char* who, const void* qkv_bf16, const void* out_bf16,
   p.tiles = (n + kTile - 1) / kTile;
   constexpr int kSmemQ = Cfg::bwd_smem(false), kSmemKV = Cfg::bwd_smem(true);
   static bool configured = false;
-  if (!configured) {
-    M3L_CUDA(cudaFuncSetAttribute(attn_long_bwd_kernel<kDh, false>, cudaFuncAttributeMaxDynamicSharedMemorySize, kSmemQ));
-    M3L_CUDA(cudaFuncSetAttribute(attn_long_bwd_kernel<kDh, true>, cudaFuncAttributeMaxDynamicSharedMemorySize, kSmemKV));
-    configured = true;
-  }
   const dim3 grid(p.tiles, heads, batch);
-  M3L_CUDA(launch_kernel(attn_long_bwd_kernel<kDh, false>, grid, dim3(320), kSmemQ, (cudaStream_t)stream, map_qkv,
-                         map_do, p));
-  M3L_CUDA(cudaGetLastError());
-  M3L_CUDA(launch_kernel(attn_long_bwd_kernel<kDh, true>, grid, dim3(320), kSmemKV, (cudaStream_t)stream, map_qkv,
-                         map_do, p));
+  if constexpr (kDrop) {
+    if (!configured) {
+      M3L_CUDA(cudaFuncSetAttribute(attn_long_drop_bwd_kernel<kDh, false>, cudaFuncAttributeMaxDynamicSharedMemorySize,
+                                    kSmemQ));
+      M3L_CUDA(cudaFuncSetAttribute(attn_long_drop_bwd_kernel<kDh, true>, cudaFuncAttributeMaxDynamicSharedMemorySize,
+                                    kSmemKV));
+      configured = true;
+    }
+    M3L_CUDA(launch_kernel(attn_long_drop_bwd_kernel<kDh, false>, grid, dim3(320), kSmemQ, (cudaStream_t)stream,
+                           map_qkv, map_do, p, dp));
+    M3L_CUDA(cudaGetLastError());
+    M3L_CUDA(launch_kernel(attn_long_drop_bwd_kernel<kDh, true>, grid, dim3(320), kSmemKV, (cudaStream_t)stream,
+                           map_qkv, map_do, p, dp));
+  } else {
+    if (!configured) {
+      M3L_CUDA(cudaFuncSetAttribute(attn_long_bwd_kernel<kDh, false>, cudaFuncAttributeMaxDynamicSharedMemorySize, kSmemQ));
+      M3L_CUDA(cudaFuncSetAttribute(attn_long_bwd_kernel<kDh, true>, cudaFuncAttributeMaxDynamicSharedMemorySize, kSmemKV));
+      configured = true;
+    }
+    M3L_CUDA(launch_kernel(attn_long_bwd_kernel<kDh, false>, grid, dim3(320), kSmemQ, (cudaStream_t)stream, map_qkv,
+                           map_do, p));
+    M3L_CUDA(cudaGetLastError());
+    M3L_CUDA(launch_kernel(attn_long_bwd_kernel<kDh, true>, grid, dim3(320), kSmemKV, (cudaStream_t)stream, map_qkv,
+                           map_do, p));
+  }
   M3L_CUDA(cudaGetLastError());
   return M3L_OK;
 }

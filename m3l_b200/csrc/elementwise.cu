@@ -11,6 +11,7 @@
 #include <type_traits>
 
 #include "common.cuh"
+#include "dropout.cuh"
 #include "m3l_internal.h"
 
 namespace m3l {
@@ -1254,6 +1255,62 @@ mse_loss_kernel(PatchSrc ps, const int64_t* __restrict__ tok_idx, int idx_ld, in
 }
 
 // ------------------------------------------------------------------------------------------
+// dropout backward: out = Z o dy (bf16, mask of dropout.cuh at plane 0), colsum[n] += sum_m out[m, n] when given
+// ------------------------------------------------------------------------------------------
+__global__ void dropout_bwd_kernel(const bf16* __restrict__ dy, int M, int N, bf16* __restrict__ out,
+                                   float* __restrict__ colsum, const DropParams dp) {
+  pdl_wait();
+  pdl_trigger();
+  // block: 32 x 8 threads; each thread owns 8 consecutive columns (one Philox call per row)
+  const int col = (blockIdx.x * 32 + threadIdx.x) * 8;
+  const uint64_t key = drop_key_load(dp.key);
+  const bool vec = (N & 7) == 0;
+  float acc[8];
+#pragma unroll
+  for (int i = 0; i < 8; ++i) acc[i] = 0.f;
+  if (col < N) {
+    for (int r = blockIdx.y * 8 + threadIdx.y; r < M; r += gridDim.y * 8) {
+      uint32_t w[4];
+      drop_words(w, key, col, r, 0, dp.site);
+      const bf16* src = dy + (size_t)r * N + col;
+      bf16* dst = out + (size_t)r * N + col;
+      float v[8];
+      if (vec) {
+        load8<bf16>(src, v);
+      } else {
+#pragma unroll
+        for (int i = 0; i < 8; ++i) v[i] = col + i < N ? __bfloat162float(src[i]) : 0.f;
+      }
+#pragma unroll
+      for (int i = 0; i < 8; ++i) {
+        v[i] = __bfloat162float(__float2bfloat16(v[i] * drop_factor(w, i, dp.thr, dp.scale)));
+        acc[i] += v[i];
+      }
+      if (vec) {
+        store8(dst, v);
+      } else {
+#pragma unroll
+        for (int i = 0; i < 8; ++i)
+          if (col + i < N) dst[i] = __float2bfloat16(v[i]);
+      }
+    }
+  }
+  if (colsum == nullptr) return;
+  __shared__ float part[8][32][8];
+#pragma unroll
+  for (int i = 0; i < 8; ++i) part[threadIdx.y][threadIdx.x][i] = acc[i];
+  __syncthreads();
+  if (threadIdx.y == 0 && col < N) {
+#pragma unroll
+    for (int i = 0; i < 8; ++i) {
+      float t = 0.f;
+      for (int y = 0; y < 8; ++y) t += part[y][threadIdx.x][i];
+      if (col + i < N) atomicAdd(colsum + col + i, t);
+    }
+  }
+}
+
+// ------------------------------------------------------------------------------------------
 // 7. column sums of a bf16 matrix: out[n] += sum_m x[m, n]   (bias gradients)
 // ------------------------------------------------------------------------------------------
 __global__ void colsum_kernel(const bf16* __restrict__ x, int M, int N, int ld, float* __restrict__ out) {
@@ -1874,6 +1931,27 @@ extern "C" int m3l_mse_loss(const m3l_patch_source* src, int batch, const int64_
     case 3: return go(mse_loss_kernel<3, 1, 6, 8, 2>, 4);     // raw uint8 frames
     default: return go(mse_loss_kernel<0, 1, 1, 8, 2>, 0);
   }
+}
+
+extern "C" int m3l_dropout_bwd(const void* dy_bf16, int rows, int cols, const int64_t* drop_key, int drop_site,
+                               float drop_p, void* out_bf16, float* colsum, void* stream) {
+  M3L_REQUIRE(dy_bf16 && out_bf16, "dropout_bwd: null pointer");
+  M3L_REQUIRE(rows >= 0 && cols >= 1, "dropout_bwd: bad shape (%d, %d)", rows, cols);
+  DropParams dp;
+  M3L_REQUIRE(drop_threshold(drop_p, &dp.thr, &dp.scale), "dropout_bwd: dropout probability %g outside [0, 1)",
+              (double)drop_p);
+  M3L_REQUIRE(drop_key != nullptr || dp.thr == 0, "dropout_bwd: null dropout key with p > 0");
+  dp.key = drop_key;
+  dp.site = (uint32_t)drop_site;
+  if (rows == 0) return M3L_OK;
+  const int gx = (cols + 255) / 256;
+  int gy = (device_sm_count() * 4 + gx - 1) / gx;
+  if (gy > (rows + 7) / 8) gy = (rows + 7) / 8;
+  if (gy > 65535) gy = 65535;
+  M3L_CUDA(launch_kernel(dropout_bwd_kernel, dim3(gx, gy), dim3(32, 8), 0, (cudaStream_t)stream,
+                         (const bf16*)dy_bf16, rows, cols, (bf16*)out_bf16, colsum, dp));
+  M3L_CUDA(cudaGetLastError());
+  return M3L_OK;
 }
 
 extern "C" int m3l_colsum(const void* x_bf16, int rows, int cols, int ld, float* out, void* stream) {

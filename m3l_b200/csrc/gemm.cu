@@ -32,6 +32,7 @@
 #include <stdlib.h>
 
 #include "common.cuh"
+#include "dropout.cuh"
 #include "m3l_internal.h"
 
 namespace m3l {
@@ -82,6 +83,9 @@ enum : int {
   EPI_F32 = 3,       // out fp32 = acc (+ bias)
   EPI_F32_RED = 4,   // out fp32 += acc  (TMA reduce-add, split-K)
   EPI_LN_BWD = 5,    // out bf16 = LayerNorm backward of acc (+ skip); dgamma / dbeta / dx column sums (N == BN == 256)
+  // dropout (training; mask Z of dropout.cuh, row / column of the output, plane 0, site drop_site):
+  EPI_GELU_DROP = 6, // out bf16 = Z o GELU(acc + bias) ; aux_out bf16 = Z o GELU'(acc + bias)
+  EPI_BF16_DROP = 7, // out bf16 = residual + Z o (acc + bias) (out2: the same values)
 };
 
 // column sums over the 32 lanes of a warp: v[c] of lane l is element (row l, column c); returns, in lane l, the sum over
@@ -187,8 +191,9 @@ gemm_bf16_kernel(const __grid_constant__ CUtensorMap map_a, const __grid_constan
     tma_prefetch_desc(&map_a);
     tma_prefetch_desc(&map_b);
     tma_prefetch_desc(&map_out);
-    if (EPI == EPI_GELU_FWD || (EPI == EPI_BF16 && p.out2 != nullptr)) tma_prefetch_desc(&map_aux);
-    if (EPI == EPI_GELU_BWD || EPI == EPI_BF16 || EPI == EPI_LN_BWD) tma_prefetch_desc(&map_side);
+    constexpr bool kPlain = EPI == EPI_BF16 || EPI == EPI_BF16_DROP;
+    if (EPI == EPI_GELU_FWD || EPI == EPI_GELU_DROP || (kPlain && p.out2 != nullptr)) tma_prefetch_desc(&map_aux);
+    if (EPI == EPI_GELU_BWD || kPlain || EPI == EPI_LN_BWD) tma_prefetch_desc(&map_side);
     if (EPI == EPI_LN_BWD) tma_prefetch_desc(&map_aux);
     for (int s = 0; s < Cfg::kStages; ++s) {
       mbar_init(&bars->full[s], 1);
@@ -473,7 +478,11 @@ gemm_bf16_kernel(const __grid_constant__ CUtensorMap map_a, const __grid_constan
     const bool has_bias = (EPI != EPI_GELU_BWD && EPI != EPI_F32_RED) && p.bias != nullptr;
     // side operand (TMA-loaded, result written in place): residual (EPI_BF16) or aux_in (GELU')
     const bool has_dot = EPI == EPI_BF16 && p.dot_out != nullptr;    // side = dot operand, output = acc
-    const bool has_side = kBufs == 2 && ((EPI == EPI_BF16 && (p.residual != nullptr || has_dot)) || EPI == EPI_GELU_BWD);
+    const bool has_side = kBufs == 2 && ((EPI == EPI_BF16 && (p.residual != nullptr || has_dot)) || EPI == EPI_GELU_BWD ||
+                                         EPI == EPI_BF16_DROP);
+    constexpr bool kDrop = EPI == EPI_GELU_DROP || EPI == EPI_BF16_DROP;
+    uint64_t dkey = 0;
+    if constexpr (kDrop) dkey = drop_key_load(p.drop_key);
     const bool want_colsum = !kF32 && p.colsum_out != nullptr;
     // fused column sums of the bf16 output (bias gradient): lane accumulates 8 columns (16-byte chunk
     // lane & 7) over the rows = (lane >> 3) mod 4 of every staged tile, in registers while this CTA
@@ -604,8 +613,18 @@ gemm_bf16_kernel(const __grid_constant__ CUtensorMap map_a, const __grid_constan
 #pragma unroll
             for (int j = 0; j < 64; ++j) v[j] = __float_as_uint(fmaxf(__uint_as_float(v[j]), 0.f));
           }
+          uint32_t keep[2];                               // dropout: keep bits of this row's 64 columns
+          if constexpr (kDrop) {
+            keep[0] = drop_keep32(dkey, gcol, row0 + lane, 0, p.drop_site, p.drop_thr);
+            keep[1] = drop_keep32(dkey, gcol + 32, row0 + lane, 0, p.drop_site, p.drop_thr);
+          }
+          if constexpr (EPI == EPI_BF16_DROP) {
+#pragma unroll
+            for (int j = 0; j < 64; ++j)
+              v[j] = __float_as_uint((keep[j >> 5] >> (j & 31)) & 1u ? __uint_as_float(v[j]) * p.drop_scale : 0.f);
+          }
           uint32_t w[32];
-          if constexpr (EPI == EPI_GELU_FWD) {
+          if constexpr (EPI == EPI_GELU_FWD || EPI == EPI_GELU_DROP) {
             // out = GELU(v); aux_out = GELU'(v) (bf16) so that the backward pass is a plain multiply
             // and never evaluates erf again (the exp(-v^2/2) is shared between the two here)
             if (p.aux_out != nullptr) {
@@ -613,6 +632,13 @@ gemm_bf16_kernel(const __grid_constant__ CUtensorMap map_a, const __grid_constan
               for (int j = 0; j < 32; ++j) {
                 f32x2 hh, gg;
                 gelu_pair(v[2 * j], v[2 * j + 1], hh, gg);
+                if constexpr (EPI == EPI_GELU_DROP) {
+                  const int c = 2 * j;
+                  const f32x2 z = f2_pack((keep[c >> 5] >> (c & 31)) & 1u ? p.drop_scale : 0.f,
+                                          (keep[c >> 5] >> ((c + 1) & 31)) & 1u ? p.drop_scale : 0.f);
+                  hh = f2_mul(hh, z);
+                  gg = f2_mul(gg, z);
+                }
                 float g0, g1;
                 f2_unpack(gg, g0, g1);
                 w[j] = pack_bf16x2(g0, g1);
@@ -624,6 +650,11 @@ gemm_bf16_kernel(const __grid_constant__ CUtensorMap map_a, const __grid_constan
               for (int j = 0; j < 32; ++j) {      // same packed evaluation as above: eval and training agree bitwise
                 f32x2 hh, gg;
                 gelu_pair(v[2 * j], v[2 * j + 1], hh, gg);
+                if constexpr (EPI == EPI_GELU_DROP) {
+                  const int c = 2 * j;
+                  hh = f2_mul(hh, f2_pack((keep[c >> 5] >> (c & 31)) & 1u ? p.drop_scale : 0.f,
+                                          (keep[c >> 5] >> ((c + 1) & 31)) & 1u ? p.drop_scale : 0.f));
+                }
                 f2_unpacku(hh, v[2 * j], v[2 * j + 1]);
               }
             }
@@ -661,7 +692,8 @@ gemm_bf16_kernel(const __grid_constant__ CUtensorMap map_a, const __grid_constan
             __syncwarp();
             if (elect_one()) {
               tma_store_2d(&map_out, sb, gcol, row0);
-              if (EPI == EPI_BF16 && p.out2 != nullptr) tma_store_2d(&map_aux, sb, gcol, row0);   // second copy of the output
+              if ((EPI == EPI_BF16 || EPI == EPI_BF16_DROP) && p.out2 != nullptr)
+                tma_store_2d(&map_aux, sb, gcol, row0);   // second copy of the output
               tma_commit_group();
             }
             if (want_colsum) add_colsum(sb, row0, r);
@@ -732,6 +764,9 @@ template <int BN>
 int launch_bn(const GemmPlan& plan, cudaStream_t stream) {
   const GemmArgs& p = plan.args;
   if (p.a_mn_major) return launch_variant<BN, true, true, EPI_F32_RED>(plan, stream);
+  if (p.drop_key != nullptr)
+    return p.act == 1 ? launch_variant<BN, false, false, EPI_GELU_DROP>(plan, stream)
+                      : launch_variant<BN, false, false, EPI_BF16_DROP>(plan, stream);
   if constexpr (BN >= 128) {
     if (plan.ws) {
       if (p.out_mode == 1) return launch_variant<BN, false, false, EPI_F32, true>(plan, stream);
@@ -793,6 +828,15 @@ int gemm_make_plan(GemmPlan* plan, const GemmArgs& args, int bn) {
   M3L_REQUIRE(p.dot_out == nullptr || (p.out_mode == 0 && p.act == 0 && p.residual == nullptr && p.N % 64 == 0 &&
                                        p.ld_dot % 8 == 0 && !p.a_mn_major),
               "gemm: the fused row-dot needs a plain bf16 output with N %% 64 == 0");
+  M3L_REQUIRE(p.drop_key != nullptr || p.drop_p == 0.f, "gemm: null dropout key with p > 0");
+  if (p.drop_key != nullptr) {
+    M3L_REQUIRE(drop_threshold(p.drop_p, &p.drop_thr, &p.drop_scale), "gemm: dropout probability %g outside [0, 1)",
+                (double)p.drop_p);
+    const bool plain = p.out_mode == 0 && !p.a_mn_major && p.ln_x == nullptr && p.dot_out == nullptr && p.splits == 1;
+    M3L_REQUIRE(plain && ((p.act == 1 && p.residual == nullptr && p.out2 == nullptr) ||
+                          (p.act == 0 && p.residual != nullptr && p.aux_out == nullptr)),
+                "gemm: dropout goes with the GELU epilogue or with bias + residual only");
+  }
   if (p.ln_x != nullptr) {
     M3L_REQUIRE(p.N == 256 && p.out_mode == 0 && !p.a_mn_major && p.splits == 1, "gemm: the LayerNorm-backward epilogue needs n == 256, bf16 output, K-major operands");
     M3L_REQUIRE(p.bias == nullptr && p.residual == nullptr && p.act == 0 && p.colsum_out == nullptr && p.dot_out == nullptr &&
@@ -843,7 +887,7 @@ int gemm_make_plan(GemmPlan* plan, const GemmArgs& args, int bn) {
   // buffered) and every CTA gets several m tiles to amortise the one-off weight load over
   // (M3L_GEMM_WS=0 disables it, for A/B measurements)
   static const bool ws_allowed = [] { const char* e = getenv("M3L_GEMM_WS"); return !(e && e[0] == '0'); }();
-  plan->ws = ws_allowed && !p.a_mn_major && kb_total <= kWsMaxKb && p.splits == 1 && bn >= 128 &&
+  plan->ws = ws_allowed && !p.a_mn_major && p.drop_key == nullptr && kb_total <= kWsMaxKb && p.splits == 1 && bn >= 128 &&
              p.residual == nullptr && p.dot_out == nullptr && p.act != 2 && p.ln_x == nullptr &&
              tiles >= 2 * device_sm_count() && tiles_n <= plan->grid;
   // decoder feed-forward forward shape (GELU + GELU' outputs, K <= 256, N % 256 == 0): dedicated kernel
@@ -894,6 +938,7 @@ extern "C" int m3l_gemm_bf16(const m3l_gemm_args* a, void* stream) {
   g.dot_side = (const m3l::bf16*)a->dot_side; g.ld_dot = a->ld_dot; g.dot_out = a->dot_out;
   g.ln_x = (const m3l::bf16*)a->ln_x; g.ln_stats = a->ln_stats; g.ln_gamma = a->ln_gamma;
   g.ln_skip = (const m3l::bf16*)a->ln_skip; g.ln_dgamma = a->ln_dgamma; g.ln_dbeta = a->ln_dbeta; g.ln_dxcol = a->ln_dxcol;
+  g.drop_key = a->drop_key; g.drop_site = (uint32_t)a->drop_site; g.drop_p = a->drop_p;
   m3l::GemmPlan plan;
   int s = m3l::gemm_make_plan(&plan, g, a->bn);
   if (s) return s;

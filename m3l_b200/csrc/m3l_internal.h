@@ -38,6 +38,13 @@ struct GemmArgs {
   float* ln_dgamma = nullptr;
   float* ln_dbeta = nullptr;
   float* ln_dxcol = nullptr;
+  // dropout epilogues (EPI_GELU_DROP / EPI_BF16_DROP; mask of dropout.cuh): key on the device, threshold / scale
+  // derived from drop_p by gemm_make_plan
+  const int64_t* drop_key = nullptr;
+  uint32_t drop_site = 0;
+  float drop_p = 0.f;
+  uint32_t drop_thr = 0;
+  float drop_scale = 1.f;
 };
 
 struct GemmPlan {

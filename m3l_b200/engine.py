@@ -188,21 +188,51 @@ class GradView:
 # --------------------------------------------------------------------------------------------
 # transformer stack (vit_pytorch.vit.Transformer without its final LayerNorm)
 # --------------------------------------------------------------------------------------------
-def stack_fwd(A: ParamArena, spec: StackSpec, x: torch.Tensor, B: int, n: int, saved: Optional[list]):
-    """x: bf16 [B*n, dim].  Returns the residual stream after the last block."""
+def p_drop(transformer) -> float:
+    """Dropout probability in force for a transformer module (vtmae.Transformer): its `dropout` in training mode,
+    0 in eval mode, as for the nn.Dropout layers of the reference."""
+    return float(transformer.p_drop) if transformer.training else 0.0
+
+
+def draw_dropout_key(device) -> torch.Tensor:
+    """The key of the dropout masks of one stack_fwd call: int64 [1] drawn on the device from torch's default CUDA
+    generator, so torch.manual_seed governs eager runs and every CUDA-graph replay draws a fresh key."""
+    return torch.randint(0, 2 ** 62, (1,), dtype=torch.int64, device=device)
+
+
+class _StackDropout:
+    """The dropout of one stack_fwd call (probability p, one key for every layer and site), kept with the saved
+    activations for stack_bwd."""
+
+    def __init__(self, key: torch.Tensor, p: float):
+        self.key, self.p = key, p
+
+    def __call__(self, layer: int, site: int) -> "ops.Dropout":
+        return ops.Dropout(self.key, (layer << 2) | site, self.p)
+
+
+def stack_fwd(A: ParamArena, spec: StackSpec, x: torch.Tensor, B: int, n: int, saved: Optional[list],
+              p_drop: float = 0.0):
+    """x: bf16 [B*n, dim].  Returns the residual stream after the last block.
+    p_drop > 0: vit_pytorch's four Dropout sites per layer (attention probabilities, to_out, after GELU, feed-forward
+    output) with the masks of csrc/dropout.cuh under a key from draw_dropout_key; callers pass their training-mode
+    probability, and 0 in eval mode.  The feed-forward block then runs as LayerNorm, GEMM + GELU, GEMM + residual,
+    and attention through the dropout kernels at every length."""
     scale = spec.dim_head ** -0.5
     M = x.shape[0]
+    drop = _StackDropout(draw_dropout_key(x.device), float(p_drop)) if p_drop > 0 else None
     for l in range(spec.depth):
         pa, pf = f"{spec.prefix}.layers.{l}.0", f"{spec.prefix}.layers.{l}.1"
         xn1, st1 = ops.layernorm_fwd(x, A.f32(pa + ".norm.weight"), A.f32(pa + ".norm.bias"),
                                      want_stats=saved is not None)
         qkv = ops.gemm(xn1, A.bf(pa + ".to_qkv.weight"))
-        o, lse = ops.mha_fwd(qkv, B, n, spec.heads, spec.dim_head, scale)
-        fused = _FUSED_MLP and ops.ln_mlp_supported(spec.dim, spec.mlp_dim)
+        o, lse = ops.mha_fwd(qkv, B, n, spec.heads, spec.dim_head, scale, dropout=drop(l, 0) if drop else None)
+        fused = _FUSED_MLP and ops.ln_mlp_supported(spec.dim, spec.mlp_dim) and drop is None
         # training keeps x_mid for the backward pass, so the attention-output GEMM writes its result twice (x_mid and
         # the buffer the fused feed-forward block then accumulates into); inference updates x_mid in place
         x_out = torch.empty_like(x) if (fused and saved is not None) else None
-        x_mid = ops.gemm(o, A.bf(pa + ".to_out.0.weight"), bias=A.f32(pa + ".to_out.0.bias"), residual=x, out2=x_out)
+        x_mid = ops.gemm(o, A.bf(pa + ".to_out.0.weight"), bias=A.f32(pa + ".to_out.0.bias"), residual=x, out2=x_out,
+                         dropout=drop(l, 1) if drop else None)
         if fused:
             # LayerNorm -> Linear -> GELU -> Linear -> + residual in ONE kernel; the [M, mlp_dim] hidden stays in
             # tensor memory (training additionally stores what the backward pass reads)
@@ -218,47 +248,65 @@ def stack_fwd(A: ParamArena, spec: StackSpec, x: torch.Tensor, B: int, n: int, s
             xn2, st2 = ops.layernorm_fwd(x_mid, A.f32(pf + ".net.0.weight"), A.f32(pf + ".net.0.bias"),
                                          want_stats=saved is not None)
             pre = torch.empty((M, spec.mlp_dim), dtype=torch.bfloat16, device=x.device) if saved is not None else None
-            h = ops.gemm(xn2, A.bf(pf + ".net.1.weight"), bias=A.f32(pf + ".net.1.bias"), act=ops.GELU_FWD, aux_out=pre)
-            x_out = ops.gemm(h, A.bf(pf + ".net.4.weight"), bias=A.f32(pf + ".net.4.bias"), residual=x_mid)
+            h = ops.gemm(xn2, A.bf(pf + ".net.1.weight"), bias=A.f32(pf + ".net.1.bias"), act=ops.GELU_FWD, aux_out=pre,
+                         dropout=drop(l, 2) if drop else None)
+            x_out = ops.gemm(h, A.bf(pf + ".net.4.weight"), bias=A.f32(pf + ".net.4.bias"), residual=x_mid,
+                             dropout=drop(l, 3) if drop else None)
         if saved is not None:
-            saved.append((x, xn1, st1, qkv, o, lse, x_mid, xn2, st2, pre, h))
+            saved.append((x, xn1, st1, qkv, o, lse, x_mid, xn2, st2, pre, h, drop))
         x = x_out
     return x
 
 
 def last_ff_bias(spec: StackSpec) -> str:
-    """Name of the bias whose gradient is the column sum of the stack-output gradient."""
+    """Name of the bias whose gradient is the column sum of the stack-output gradient (without dropout)."""
     return f"{spec.prefix}.layers.{spec.depth - 1}.1.net.4.bias"
+
+
+def stack_dx_colsum(G: GradView, spec: StackSpec, saved: list) -> Optional[torch.Tensor]:
+    """Where the producer of stack_bwd's dx accumulates the column sums of dx: the gradient of the last feed-forward
+    bias, G(last_ff_bias(spec)).  None when the forward applied dropout: that gradient is then the column sum of the
+    dropped-out dx, which stack_bwd accumulates itself."""
+    return None if saved[-1][-1] is not None else G(last_ff_bias(spec))
 
 
 def stack_bwd(A: ParamArena, G: GradView, spec: StackSpec, dx: torch.Tensor, B: int, n: int, saved: list):
     """dx: bf16 [B*n, dim] gradient w.r.t. the stack output.  Returns the gradient w.r.t. its input.
     The producer of dx (the final-LayerNorm backward) must already have accumulated its column sums
-    into G(last_ff_bias(spec)) (dx_colsum= of ops.layernorm_bwd)."""
+    into stack_dx_colsum(G, spec, saved) when that is not None (dx_colsum= of ops.layernorm_bwd)."""
     scale = spec.dim_head ** -0.5
     M = dx.shape[0]
     fork = WgradFork(A.device)
     for l in reversed(range(spec.depth)):
         pa, pf = f"{spec.prefix}.layers.{l}.0", f"{spec.prefix}.layers.{l}.1"
-        x, xn1, st1, qkv, o, lse, x_mid, xn2, st2, pre, h = saved[l]
-        # ---- feed-forward branch: x_out = x_mid + W2 gelu(W1 LN2(x_mid) + b1) + b2
-        fork.wgrad(dx, h, G(pf + ".net.4.weight"))
-        dpre = ops.gemm(dx, A.bf_t(pf + ".net.4.weight"), act=ops.GELU_BWD, aux_in=pre,
+        x, xn1, st1, qkv, o, lse, x_mid, xn2, st2, pre, h, drop = saved[l]
+        # ---- feed-forward branch: x_out = x_mid + Z3 o (W2 h + b2), h = Z2 o gelu(W1 LN2(x_mid) + b1) (Z = 1 without
+        # dropout); pre holds Z2 o gelu', so the GELU' product below is the backward through Z2 as well
+        dy = dx
+        if drop is not None:
+            dy = ops.dropout_bwd(dx, drop(l, 3), colsum=G(pf + ".net.4.bias"))
+        fork.wgrad(dy, h, G(pf + ".net.4.weight"))
+        dpre = ops.gemm(dy, A.bf_t(pf + ".net.4.weight"), act=ops.GELU_BWD, aux_in=pre,
                         colsum_out=G(pf + ".net.1.bias"))
         fork.wgrad(dpre, xn2, G(pf + ".net.1.weight"))
         dx_mid = _dgrad_ln_bwd(dpre, A.bf_t(pf + ".net.1.weight"), x_mid, st2, A.f32(pf + ".net.0.weight"),
-                               G(pf + ".net.0.weight"), G(pf + ".net.0.bias"), dx, G(pa + ".to_out.0.bias"))
-        # ---- attention branch: x_mid = x + Wo attn(Wqkv LN1(x)) + bo
-        fork.wgrad(dx_mid, o, G(pa + ".to_out.0.weight"))
+                               G(pf + ".net.0.weight"), G(pf + ".net.0.bias"), dx,
+                               G(pa + ".to_out.0.bias") if drop is None else None)
+        # ---- attention branch: x_mid = x + Z1 o (Wo attn(Wqkv LN1(x)) + bo), attention probabilities dropped by Z0
+        dy_mid = dx_mid
+        if drop is not None:
+            dy_mid = ops.dropout_bwd(dx_mid, drop(l, 1), colsum=G(pa + ".to_out.0.bias"))
+        fork.wgrad(dy_mid, o, G(pa + ".to_out.0.weight"))
         # dO, and in the same epilogue delta = rowsum(dO * O) per head (dim_head == 64 == one epilogue round)
         delta = torch.empty((M, spec.heads), dtype=torch.float32, device=dx.device) if spec.dim_head == 64 else None
-        do = ops.gemm(dx_mid, A.bf_t(pa + ".to_out.0.weight"), dot_side=o if delta is not None else None, dot_out=delta)
-        dqkv = ops.mha_bwd(qkv, o, do, lse, B, n, spec.heads, spec.dim_head, scale, delta=delta)
+        do = ops.gemm(dy_mid, A.bf_t(pa + ".to_out.0.weight"), dot_side=o if delta is not None else None, dot_out=delta)
+        dqkv = ops.mha_bwd(qkv, o, do, lse, B, n, spec.heads, spec.dim_head, scale, delta=delta,
+                           dropout=drop(l, 0) if drop else None)
         fork.wgrad(dqkv, xn1, G(pa + ".to_qkv.weight"))
-        prev_bias = G(f"{spec.prefix}.layers.{l - 1}.1.net.4.bias") if l > 0 else None
+        prev_bias = G(f"{spec.prefix}.layers.{l - 1}.1.net.4.bias") if (l > 0 and drop is None) else None
         dx_in = _dgrad_ln_bwd(dqkv, A.bf_t(pa + ".to_qkv.weight"), x, st1, A.f32(pa + ".norm.weight"),
                               G(pa + ".norm.weight"), G(pa + ".norm.bias"), dx_mid, prev_bias)
-        fork.join()          # this layer's wgrad operands (dx, dpre, dx_mid, dqkv) die below
+        fork.join()          # this layer's wgrad operands (dy, dpre, dy_mid, dqkv) die below
         dx = dx_in
     return dx
 
@@ -601,7 +649,7 @@ def mae_forward(model, x: Dict[str, torch.Tensor], noise: torch.Tensor, geo: Geo
     else:
         x0 = _embed_fwd(model, A, geo, tabs, x, B, unmasked, True, emb_saved, unmasked32=unmasked32)
     enc_saved = [] if training else None
-    xe = stack_fwd(A, model.enc_spec, x0, B, geo.nv, enc_saved)
+    xe = stack_fwd(A, model.enc_spec, x0, B, geo.nv, enc_saved, p_drop=p_drop(model.encoder.transformer))
     enc_out, st_enc = ops.layernorm_fwd(xe, A.f32("encoder.transformer.norm.weight"), A.f32("encoder.transformer.norm.bias"),
                                         want_stats=training)
     if model.has_enc_to_dec:
@@ -706,7 +754,7 @@ def mae_backward_encoder_stack(model, ctx, gflat: torch.Tensor):
         denc = dd
     dxe = ops.layernorm_bwd(denc, ctx["xe"], ctx["st_enc"], A.f32("encoder.transformer.norm.weight"),
                             dgamma=G("encoder.transformer.norm.weight"), dbeta=G("encoder.transformer.norm.bias"),
-                            dx_colsum=G(last_ff_bias(model.enc_spec)))
+                            dx_colsum=stack_dx_colsum(G, model.enc_spec, ctx["enc"]))
     return stack_bwd(A, G, model.enc_spec, dxe, B, geo.nv, ctx["enc"])
 
 
@@ -741,7 +789,7 @@ def embeddings_forward(model, x, geo: Geometry, B: int, training: bool):
     else:
         x0 = _embed_fwd(model, A, geo, tabs, x, B, None, False, emb_saved)
     enc_saved = [] if training else None
-    xe = stack_fwd(A, model.enc_spec, x0, B, geo.n, enc_saved)
+    xe = stack_fwd(A, model.enc_spec, x0, B, geo.n, enc_saved, p_drop=p_drop(model.encoder.transformer))
     out, st = ops.layernorm_fwd(xe, A.f32("encoder.transformer.norm.weight"), A.f32("encoder.transformer.norm.bias"),
                                 want_stats=training)
     ctx = dict(geo=geo, B=B, tabs=tabs, emb=emb_saved, enc=enc_saved, xe=xe, st=st, tokens_all=x0) if training else None
@@ -756,7 +804,7 @@ def embeddings_backward(model, ctx, dout: torch.Tensor, gflat: torch.Tensor, ext
     geo, B, tabs = ctx["geo"], ctx["B"], ctx["tabs"]
     dxe = ops.layernorm_bwd(dout, ctx["xe"], ctx["st"], A.f32("encoder.transformer.norm.weight"),
                             dgamma=G("encoder.transformer.norm.weight"), dbeta=G("encoder.transformer.norm.bias"),
-                            dx_colsum=G(last_ff_bias(model.enc_spec)))
+                            dx_colsum=stack_dx_colsum(G, model.enc_spec, ctx["enc"]))
     dx0 = stack_bwd(A, G, model.enc_spec, dxe, B, geo.n, ctx["enc"])
     if extra_token_grad is not None:
         ops.row_scatter_add(extra_token_grad[0], extra_token_grad[1], B, geo.n, dx0)

@@ -6,7 +6,7 @@ C-ABI and returns torch tensors.  torch is only the allocator / stream provider 
 from __future__ import annotations
 
 import ctypes as C
-from typing import Optional
+from typing import NamedTuple, Optional
 
 import torch
 
@@ -16,6 +16,22 @@ from ._lib import GemmArgs, check, current_stream, ptr
 GELU_FWD = 1
 GELU_BWD = 2
 RELU = 3
+
+
+class Dropout(NamedTuple):
+    """One dropout site of a training pass: key int64 [1] on the device, site = (layer << 2) | s (s = 0 attention
+    probabilities, 1 attention output, 2 after GELU, 3 feed-forward output), p in [0, 1).  The mask is the
+    counter-based one of csrc/dropout.cuh (include/m3l_b200.h)."""
+    key: torch.Tensor
+    site: int
+    p: float
+
+
+def _drop_args(d: Optional[Dropout]):
+    if d is None:
+        return C.c_void_p(0), 0, C.c_float(0.0)
+    assert d.key.dtype == torch.int64 and d.key.is_cuda and d.key.numel() >= 1
+    return ptr(d.key), int(d.site), C.c_float(d.p)
 
 
 _WS = {}
@@ -45,11 +61,14 @@ def gemm(a: torch.Tensor, b: torch.Tensor, *, mn_major: bool = False, out: Optio
          aux_out: Optional[torch.Tensor] = None, aux_in: Optional[torch.Tensor] = None,
          alpha: float = 1.0, colsum_out: Optional[torch.Tensor] = None,
          dot_side: Optional[torch.Tensor] = None, dot_out: Optional[torch.Tensor] = None,
-         out2: Optional[torch.Tensor] = None, ln_bwd: Optional[dict] = None) -> torch.Tensor:
+         out2: Optional[torch.Tensor] = None, ln_bwd: Optional[dict] = None,
+         dropout: Optional[Dropout] = None) -> torch.Tensor:
     """out[m, n] = epilogue(alpha * sum_k A[m, k] B[n, k]).
 
     mn_major=False: a is [M, K], b is [N, K] (nn.Linear forward: x @ W.T).
     mn_major=True : a is [K, M], b is [K, N] (wgrad: a.T @ b), optionally split-K + accumulate.
+    dropout: with act=GELU_FWD, out = Z o GELU and aux_out = Z o GELU'; with a residual (act 0),
+    out = residual + Z o (acc + bias).  Other epilogues reject it.
     """
     _req_cuda(a, b, out, bias, residual, aux_out, aux_in)
     assert a.dtype == torch.bfloat16 and b.dtype == torch.bfloat16
@@ -101,6 +120,8 @@ def gemm(a: torch.Tensor, b: torch.Tensor, *, mn_major: bool = False, out: Optio
         assert sk is None or (sk.shape == (M, N) and sk.dtype == torch.bfloat16 and sk.is_contiguous())
         args.ln_x, args.ln_stats, args.ln_gamma, args.ln_skip = ptr(x), ptr(st), ptr(gm), ptr(sk)
         args.ln_dgamma, args.ln_dbeta, args.ln_dxcol = ptr(ln_bwd["dgamma"]), ptr(ln_bwd["dbeta"]), ptr(ln_bwd.get("dx_colsum"))
+    if dropout is not None:
+        args.drop_key, args.drop_site, args.drop_p = _drop_args(dropout)
     check(_lib.load().m3l_gemm_bf16(C.byref(args), current_stream()), "m3l_gemm_bf16")
     return out
 
@@ -485,6 +506,50 @@ def attention_dh_bwd(qkv, out, dout, lse, batch, n, heads, dim_head, scale, *, d
     return dqkv
 
 
+def attention_dropout_fwd(qkv, batch, n, heads, dim_head, scale, dropout: Dropout, *, out=None, lse=None):
+    """attention_long_fwd / attention_dh_fwd with dropout on the attention probabilities (csrc/attention_dropout.cu),
+    dim_head 32, 64 or 128, any n >= 1.  lse is that of the undropped scores."""
+    _req_cuda(qkv)
+    inner = heads * dim_head
+    assert qkv.dtype == torch.bfloat16 and qkv.is_contiguous() and qkv.shape == (batch * n, 3 * inner)
+    if out is None:
+        out = torch.empty((batch * n, inner), dtype=torch.bfloat16, device=qkv.device)
+    if lse is None:
+        lse = torch.empty((batch, heads, n), dtype=torch.float32, device=qkv.device)
+    check(_lib.load().m3l_attention_dropout_fwd(ptr(qkv), batch, n, heads, dim_head, C.c_float(scale),
+                                                *_drop_args(dropout), ptr(out), ptr(lse), current_stream()),
+          "m3l_attention_dropout_fwd")
+    return out, lse
+
+
+def attention_dropout_bwd(qkv, out, dout, lse, batch, n, heads, dim_head, scale, dropout: Dropout, *, dqkv=None,
+                          delta=None):
+    """Backward of attention_dropout_fwd (same mask; delta optional as in attention_long_bwd)."""
+    _req_cuda(qkv, out, dout, lse, dqkv, delta)
+    if dqkv is None:
+        dqkv = torch.empty_like(qkv)
+    assert dout.is_contiguous() and out.is_contiguous()
+    assert delta is None or (delta.dtype == torch.float32 and delta.is_contiguous() and delta.shape == (batch * n, heads))
+    check(_lib.load().m3l_attention_dropout_bwd(ptr(qkv), ptr(out), ptr(dout), ptr(lse), ptr(delta), batch, n, heads,
+                                                dim_head, C.c_float(scale), *_drop_args(dropout), ptr(dqkv),
+                                                current_stream()), "m3l_attention_dropout_bwd")
+    return dqkv
+
+
+def dropout_bwd(dy, dropout: Dropout, *, out=None, colsum=None):
+    """out = Z o dy (bf16 [rows, cols], contiguous): the backward of a dropout site of the GEMM epilogues;
+    colsum (fp32 [cols]) += column sums of out when given (the bias gradient of the Linear before the dropout)."""
+    _req_cuda(dy, out, colsum)
+    assert dy.dtype == torch.bfloat16 and dy.is_contiguous() and dy.dim() == 2
+    if out is None:
+        out = torch.empty_like(dy)
+    assert out.shape == dy.shape and out.dtype == torch.bfloat16 and out.is_contiguous()
+    assert colsum is None or (colsum.dtype == torch.float32 and colsum.numel() == dy.shape[1])
+    check(_lib.load().m3l_dropout_bwd(ptr(dy), dy.shape[0], dy.shape[1], *_drop_args(dropout), ptr(out), ptr(colsum),
+                                      current_stream()), "m3l_dropout_bwd")
+    return out
+
+
 # longest sequence the single-CTA kernels of csrc/attention.cu take; above it csrc/attention_long.cu runs
 SHORT_ATTENTION_MAX_N = 256
 # head widths with kernels: 64 (attention.cu / attention_long.cu), 32 and 128 (attention_dh.cu)
@@ -499,16 +564,23 @@ def _mha_kernels(n, dim_head):
     return attention_long_fwd, attention_long_bwd
 
 
-def mha_fwd(qkv, batch, n, heads, dim_head, scale, *, out=None, lse=None):
+def mha_fwd(qkv, batch, n, heads, dim_head, scale, *, out=None, lse=None, dropout: Optional[Dropout] = None):
     """Multi-head attention forward for any sequence length.  64-wide heads: attention_fwd up to
-    SHORT_ATTENTION_MAX_N tokens, attention_long_fwd above; 32- and 128-wide heads: attention_dh_fwd for every n.
+    SHORT_ATTENTION_MAX_N tokens, attention_long_fwd above; 32- and 128-wide heads: attention_dh_fwd for every n;
+    with dropout, attention_dropout_fwd for every n and width.
     The one place the model code picks between the kernel families."""
+    if dropout is not None:
+        return attention_dropout_fwd(qkv, batch, n, heads, dim_head, scale, dropout, out=out, lse=lse)
     f = _mha_kernels(n, dim_head)[0]
     return f(qkv, batch, n, heads, dim_head, scale, out=out, lse=lse)
 
 
-def mha_bwd(qkv, out, dout, lse, batch, n, heads, dim_head, scale, *, dqkv=None, delta=None):
-    """Backward of mha_fwd (same selection by n and dim_head)."""
+def mha_bwd(qkv, out, dout, lse, batch, n, heads, dim_head, scale, *, dqkv=None, delta=None,
+            dropout: Optional[Dropout] = None):
+    """Backward of mha_fwd (same selection by n, dim_head and dropout)."""
+    if dropout is not None:
+        return attention_dropout_bwd(qkv, out, dout, lse, batch, n, heads, dim_head, scale, dropout, dqkv=dqkv,
+                                     delta=delta)
     f = _mha_kernels(n, dim_head)[1]
     return f(qkv, out, dout, lse, batch, n, heads, dim_head, scale, dqkv=dqkv, delta=delta)
 

@@ -17,6 +17,8 @@ What each op stands in for in the reference (paths under /root/reference):
   m3l::attention_fwd / attention_bwd      softmax(q k^T / sqrt(d)) v of vit_pytorch.Attention, fused (n <= 256)
   m3l::attention_long_fwd / attention_long_bwd   the same for any sequence length (online softmax over key tiles)
   m3l::attention_dh_fwd / attention_dh_bwd       the same for 32- and 128-wide heads, any sequence length
+  m3l::attention_dropout_fwd / attention_dropout_bwd   the same with Attention.dropout on the probabilities (training)
+  m3l::dropout_bwd    backward of a Dropout applied in a GEMM epilogue (FeedForward / Attention.to_out Dropout)
   m3l::ln_mlp_fwd / ln_mlp_bwd            x + FeedForward(x) of vit_pytorch.Transformer as one kernel each way
   m3l::mask_indices   torch.rand(...).argsort() split into masked / unmasked (models/pretrain_models.py:229-248)
   m3l::patch_layernorm                    Rearrange('b c (h p1) (w p2) -> b (h w) (p1 p2 c)') + gather + LayerNorm (:164-198,766-779)
@@ -177,6 +179,45 @@ def _attn_dh_bwd(qkv: Tensor, out: Tensor, dout: Tensor, lse: Tensor, batch: int
 
 _define("attention_dh_bwd(Tensor qkv, Tensor out, Tensor dout, Tensor lse, int batch, int n, int heads, int dim_head, "
         "float scale) -> Tensor", _attn_dh_bwd, _attn_bwd_fake)
+
+
+def _attn_dropout_fwd(qkv: Tensor, batch: int, n: int, heads: int, dim_head: int, scale: float, key: Tensor, site: int,
+                      p: float) -> Tuple[Tensor, Tensor]:
+    return ops.attention_dropout_fwd(qkv.contiguous(), batch, n, heads, dim_head, scale, ops.Dropout(key, site, p))
+
+
+def _attn_dropout_fwd_fake(qkv, batch, n, heads, dim_head, scale, key, site, p):
+    return _attn_fwd_fake(qkv, batch, n, heads, dim_head, scale)
+
+
+_define("attention_dropout_fwd(Tensor qkv, int batch, int n, int heads, int dim_head, float scale, Tensor key, int site, "
+        "float p) -> (Tensor, Tensor)", _attn_dropout_fwd, _attn_dropout_fwd_fake)
+
+
+def _attn_dropout_bwd(qkv: Tensor, out: Tensor, dout: Tensor, lse: Tensor, batch: int, n: int, heads: int, dim_head: int,
+                      scale: float, key: Tensor, site: int, p: float) -> Tensor:
+    return ops.attention_dropout_bwd(qkv.contiguous(), out.contiguous(), dout.contiguous(), lse.contiguous(), batch, n,
+                                     heads, dim_head, scale, ops.Dropout(key, site, p))
+
+
+def _attn_dropout_bwd_fake(qkv, out, dout, lse, batch, n, heads, dim_head, scale, key, site, p):
+    return _attn_bwd_fake(qkv, out, dout, lse, batch, n, heads, dim_head, scale)
+
+
+_define("attention_dropout_bwd(Tensor qkv, Tensor out, Tensor dout, Tensor lse, int batch, int n, int heads, "
+        "int dim_head, float scale, Tensor key, int site, float p) -> Tensor", _attn_dropout_bwd, _attn_dropout_bwd_fake)
+
+
+def _dropout_bwd(dy: Tensor, key: Tensor, site: int, p: float) -> Tensor:
+    return ops.dropout_bwd(dy.contiguous(), ops.Dropout(key, site, p))
+
+
+def _dropout_bwd_fake(dy, key, site, p):
+    torch._check(dy.dim() == 2 and dy.dtype == torch.bfloat16, lambda: "dropout_bwd: dy [rows, cols] bf16")
+    return dy.new_empty(dy.shape)
+
+
+_define("dropout_bwd(Tensor dy, Tensor key, int site, float p) -> Tensor", _dropout_bwd, _dropout_bwd_fake)
 
 
 # ---------------------------------------------------------------------------------------------- fused feed-forward block

@@ -165,7 +165,7 @@ class FusedTrainer:
                 self._phase_c(ranges)
             A._version_seen = A.version()
             return box["loss"].reshape(())
-        key = (geo.use_vision, geo.nt, B, input_signature(xs))
+        key = (geo.use_vision, geo.nt, B, input_signature(xs), engine.p_drop(model.encoder.transformer))
         g = self._graphs.get(key)
         if g is None:
             while len(self._graphs) >= self._MAX_GRAPHS:       # each capture owns a full activation pool

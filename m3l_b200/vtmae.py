@@ -83,8 +83,6 @@ class Transformer(nn.Module):
 
     def forward(self, x):
         """x: (B, n, dim) -> (B, n, dim); differentiable w.r.t. x and the parameters."""
-        if self.p_drop > 0 and self.training:
-            raise M3LError("dropout > 0 in training mode is not supported by the fused kernels")
         A = self._own_arena()
         spec = engine.StackSpec("t", self.dim, self.depth, self.heads, self.dim_head, self.mlp_dim)
         names = list(A.names)
@@ -98,7 +96,7 @@ class _TransformerFn(torch.autograd.Function):
         need = any(ctx.needs_input_grad)
         xb = x.detach().reshape(B * n, D).to(torch.bfloat16).contiguous()
         saved = [] if need else None
-        xe = engine.stack_fwd(A, spec, xb, B, n, saved)
+        xe = engine.stack_fwd(A, spec, xb, B, n, saved, p_drop=engine.p_drop(mod))
         out, st = ops.layernorm_fwd(xe, A.f32("t.norm.weight"), A.f32("t.norm.bias"), want_stats=need)
         ctx.c = (A, spec, saved, xe, st, B, n, D)
         return out.float().reshape(B, n, D)
@@ -110,7 +108,7 @@ class _TransformerFn(torch.autograd.Function):
         G = engine.GradView(A, gflat)
         dout = gout.reshape(B * n, D).to(torch.bfloat16).contiguous()
         dxe = ops.layernorm_bwd(dout, xe, st, A.f32("t.norm.weight"), dgamma=G("t.norm.weight"), dbeta=G("t.norm.bias"),
-                                dx_colsum=G(engine.last_ff_bias(spec)))
+                                dx_colsum=engine.stack_dx_colsum(G, spec, saved))
         dx = engine.stack_bwd(A, G, spec, dxe, B, n, saved)
         return (None, None, None, dx.float().reshape(B, n, D), *[A.view(gflat, nm) for nm in A.names])
 
@@ -363,7 +361,7 @@ class VTMAE(nn.Module):
         live = self.live_param_names(geo, True)
         params = [A.params[k] for k in live]
         if self.use_cuda_graph and torch.is_grad_enabled() and any(p.requires_grad for p in params):
-            key = ("mae", geo.use_vision, geo.nt, B, input_signature(xs))
+            key = ("mae", geo.use_vision, geo.nt, B, input_signature(xs), engine.p_drop(self.encoder.transformer))
             # The graph entry owns ONE set of saved activations.  If the previous replayed forward of this shape has
             # not been back-propagated yet (two forwards before a backward: SAC with a shared extractor, gradient
             # accumulation over two losses), this call takes the eager autograd path, which owns its activations.
@@ -384,7 +382,7 @@ class VTMAE(nn.Module):
         params = [A.params[k] for k in live]
         if self.use_cuda_graph and torch.is_grad_enabled() and any(p.requires_grad for p in params):
             cache = self.__dict__.setdefault("_mae_graphs", {})
-            key = ("emb", geo.use_vision, geo.nt, B, input_signature(xs))
+            key = ("emb", geo.use_vision, geo.nt, B, input_signature(xs), engine.p_drop(self.encoder.transformer))
             ent = cache.get(key)
             if _entry_free(ent):                  # else: previous forward not back-propagated yet -> eager path
                 if ent is None:
@@ -562,7 +560,8 @@ class MAEExtractor(_ExtractorBase):
         if noise is None:
             noise = torch.rand(B, geo.n, device=dev)
         noise = noise.to(device=dev, dtype=torch.float32).contiguous()
-        key = ("joint",) + tuple((k, tuple(v.shape), v.dtype) for k, v in sorted(obs.items())) + (id(A), id(Av))
+        key = ("joint",) + tuple((k, tuple(v.shape), v.dtype) for k, v in sorted(obs.items())) + (id(A), id(Av)) + \
+              self._p_drops()
         cache = self.__dict__.setdefault("_graphs", {})
         ent = cache.get(key)
         if not _entry_free(ent):
@@ -590,7 +589,7 @@ class MAEExtractor(_ExtractorBase):
         A = mae._sync()
         Av = self.vit_layer.transformer._own_arena()
         key = ("grad",) + tuple((k, tuple(v.shape), v.dtype) for k, v in sorted(obs.items())) + \
-              (bool(self.vision_only_control), id(A), id(Av))
+              (bool(self.vision_only_control), id(A), id(Av)) + self._p_drops()
         cache = self.__dict__.setdefault("_graphs", {})
         ent = cache.get(key)
         if not _entry_free(ent):                  # previous forward of this shape not back-propagated yet
@@ -616,6 +615,7 @@ class MAEExtractor(_ExtractorBase):
         A = mae._sync()                                           # bf16 shadows current (outside the graph)
         Av = self.vit_layer.transformer._own_arena()
         key = key + (id(A), id(Av))                               # a re-created arena invalidates captured pointers
+        key = key + self._p_drops()                               # the dropout of a graph is fixed at capture
         ent = cache.get(key)
         if ent is None:
             static_in = {k: v.clone() for k, v in obs.items()}
@@ -655,11 +655,13 @@ class MAEExtractor(_ExtractorBase):
         mae.train()                                               # get_embeddings(eval=False) side effect (:590-593)
         A = mae._sync()
         xs, geo, B = mae._prep_inputs(vt, True, not self.vision_only_control)
-        tr = self.vit_layer.transformer
-        if tr.p_drop > 0 and tr.training:
-            raise M3LError("dropout > 0 in training mode is not supported by the fused kernels")
-        Av = tr._own_arena()
+        Av = self.vit_layer.transformer._own_arena()
         return xs, geo, B, A, Av
+
+    def _p_drops(self):
+        """Dropout probabilities in force for the MAE encoder and the extra block (part of every graph key).  The MAE
+        runs in training mode here (get_embeddings(eval=False) in the reference), so its encoder dropout applies."""
+        return engine.p_drop(self.mae_model.encoder.transformer), engine.p_drop(self.vit_layer.transformer)
 
 
 class _ExtractorFn(torch.autograd.Function):
@@ -671,7 +673,7 @@ class _ExtractorFn(torch.autograd.Function):
         emb, c = engine.embeddings_forward(mae, xs, geo, B, training=need)
         spec = engine.StackSpec("t", tr.dim, tr.depth, tr.heads, tr.dim_head, tr.mlp_dim)
         saved = [] if need else None
-        xe = engine.stack_fwd(Av, spec, emb, B, geo.n, saved)
+        xe = engine.stack_fwd(Av, spec, emb, B, geo.n, saved, p_drop=engine.p_drop(tr))
         y, st = ops.layernorm_fwd(xe, Av.f32("t.norm.weight"), Av.f32("t.norm.bias"), want_stats=need)
         out = ops.token_mean_fwd(y, B, geo.n)
         ctx.c = (mae, Av, spec, c, saved, xe, st, B, geo.n, live, vit_names)
@@ -685,7 +687,7 @@ class _ExtractorFn(torch.autograd.Function):
         gv = Av.new_grad_buffer()
         Gv = engine.GradView(Av, gv)
         dxe = ops.layernorm_bwd(dy, xe, st, Av.f32("t.norm.weight"), dgamma=Gv("t.norm.weight"), dbeta=Gv("t.norm.bias"),
-                                dx_colsum=Gv(engine.last_ff_bias(spec)))
+                                dx_colsum=engine.stack_dx_colsum(Gv, spec, saved))
         demb = engine.stack_bwd(Av, Gv, spec, dxe, B, n, saved)
         gm = A.new_grad_buffer()
         engine.embeddings_backward(mae, c, demb, gm)
@@ -707,7 +709,7 @@ def _capture_extractor_graphs(ext, obs):
         xs, geo, B, _, _ = ext._prep(dict(ent.xs))
         emb, c = engine.embeddings_forward(mae, xs, geo, B, training=True)
         saved = []
-        xe = engine.stack_fwd(Av, spec, emb, B, geo.n, saved)
+        xe = engine.stack_fwd(Av, spec, emb, B, geo.n, saved, p_drop=engine.p_drop(tr))
         y, st = ops.layernorm_fwd(xe, Av.f32("t.norm.weight"), Av.f32("t.norm.bias"), want_stats=True)
         ent.loss = ops.token_mean_fwd(y, B, geo.n)
         ent.ctx = (c, saved, xe, st, B, geo.n)
@@ -719,7 +721,7 @@ def _capture_extractor_graphs(ext, obs):
         Gv = engine.GradView(Av, ent.gflat2)
         dy = ops.token_mean_bwd(ent.gout, B, n)
         dxe = ops.layernorm_bwd(dy, xe, st, Av.f32("t.norm.weight"), dgamma=Gv("t.norm.weight"), dbeta=Gv("t.norm.bias"),
-                                dx_colsum=Gv(engine.last_ff_bias(spec)))
+                                dx_colsum=engine.stack_dx_colsum(Gv, spec, saved))
         demb = engine.stack_bwd(Av, Gv, spec, dxe, B, n, saved)
         engine.embeddings_backward(mae, c, demb, ent.gflat)
 
@@ -780,7 +782,7 @@ def _joint_forward(ext, xs, noise, geo, B, gflat_m):
     loss_acc, cm = engine.mae_forward(mae, xs, noise, geo, training=True, gflat=gflat_m, tokens_all=c["tokens_all"])
     spec = engine.StackSpec("t", tr.dim, tr.depth, tr.heads, tr.dim_head, tr.mlp_dim)
     saved = []
-    xe = engine.stack_fwd(Av, spec, emb, B, geo.n, saved)
+    xe = engine.stack_fwd(Av, spec, emb, B, geo.n, saved, p_drop=engine.p_drop(tr))
     y, st = ops.layernorm_fwd(xe, Av.f32("t.norm.weight"), Av.f32("t.norm.bias"), want_stats=True)
     feats = ops.token_mean_fwd(y, B, geo.n)
     return loss_acc, feats, (c, cm, spec, saved, xe, st, B, geo.n)
@@ -794,7 +796,7 @@ def _joint_backward(ext, ctx, g_loss, g_feats, gflat, gflat_m, gflat2):
     Gv = engine.GradView(Av, gflat2)
     dy = ops.token_mean_bwd(g_feats, B, n)
     dxe = ops.layernorm_bwd(dy, xe, st, Av.f32("t.norm.weight"), dgamma=Gv("t.norm.weight"), dbeta=Gv("t.norm.bias"),
-                            dx_colsum=Gv(engine.last_ff_bias(spec)))
+                            dx_colsum=engine.stack_dx_colsum(Gv, spec, saved))
     demb = engine.stack_bwd(Av, Gv, spec, dxe, B, n, saved)
     engine.mae_backward_decoder(mae, cm, gflat_m)
     dx0 = engine.mae_backward_encoder(mae, cm, gflat_m)

@@ -138,9 +138,6 @@ class VTT(nn.Module):
     def forward_features(self, x, masks: Optional[List[torch.Tensor]] = None):
         """x: dict(image (B,C,H,W), tactile1, tactile2) fp32 CUDA; masks: list of (B, K) keep-index tensors shared
         by the three modalities (tactile_ssl/utils/__init__.py:25-36) -> the reference's dict of (len(masks)*B, ., D)."""
-        tr = self.transformer
-        if tr.p_drop > 0 and self.training:
-            raise M3LError("dropout > 0 in training mode is not supported by the fused kernels")
         A = self._own_arena()
         maps = []
         for k in _KEYS:
@@ -198,7 +195,7 @@ class _VTTFn(torch.autograd.Function):
         tr = mod.transformer
         spec = engine.StackSpec("transformer", tr.dim, tr.depth, tr.heads, tr.dim_head, tr.mlp_dim)
         saved = [] if need else None
-        xe = engine.stack_fwd(A, spec, x0, Beff, n, saved)
+        xe = engine.stack_fwd(A, spec, x0, Beff, n, saved, p_drop=engine.p_drop(tr))
         xt, st_t = ops.layernorm_fwd(xe, A.f32("transformer.norm.weight"), A.f32("transformer.norm.bias"), want_stats=need)
         xn, st_n = ops.layernorm_fwd(xt, A.f32("norm.weight"), A.f32("norm.bias"), want_stats=need, eps=1e-6)
         ctx.c = (A, spec, emb_saved, saved, xe, st_t, xt, st_n, Beff, n, D, R, names)
@@ -213,7 +210,8 @@ class _VTTFn(torch.autograd.Function):
         skip = g_pre.reshape(Beff * n, D).to(torch.bfloat16).contiguous()
         dxt = ops.layernorm_bwd(dn, xt, st_n, A.f32("norm.weight"), dgamma=G("norm.weight"), dbeta=G("norm.bias"), skip=skip)
         dxe = ops.layernorm_bwd(dxt, xe, st_t, A.f32("transformer.norm.weight"), dgamma=G("transformer.norm.weight"),
-                                dbeta=G("transformer.norm.bias"), dx_colsum=G(engine.last_ff_bias(spec)))
+                                dbeta=G("transformer.norm.bias"),
+                                dx_colsum=engine.stack_dx_colsum(G, spec, saved))
         dx0 = engine.stack_bwd(A, G, spec, dxe, Beff, n, saved)
         if R:
             G("register_tokens").copy_(dx0.view(Beff, n, D)[:, :R].float().sum(0, keepdim=True))
