@@ -391,6 +391,16 @@ int m3l_cast_bf16(const float* src, void* dst_bf16, size_t count, void* stream);
 int m3l_transpose_cast_bf16(const float* src_base, void* dst_base_bf16, const m3l_matrix_desc* descs_dev,
                             int count, void* stream);
 
+/* LayerScale fold of DINOv2 fine-tuning (csrc/layerscale.cu).  fold: wf = bf16(gamma_r * w[r, c]) [rows, cols],
+ * wf_t its transpose [cols, rows] (nullable), bf = gamma o b fp32 (nullable); gamma == NULL casts w unscaled.
+ * The rounding is torch's (fp32 product, then round-to-nearest-even bf16).
+ * unfold: from the fp32 gradients dwf / dbf of the folded Linear, dw = gamma o dwf, db = gamma o dbf,
+ * dgamma[r] = sum_c w[r, c] dwf[r, c] + b[r] dbf[r] (all written, not accumulated). */
+int m3l_layerscale_fold(const float* w, const float* b, const float* gamma, int rows, int cols, void* wf_bf16,
+                        void* wf_t_bf16, float* bf, void* stream);
+int m3l_layerscale_unfold(const float* dwf, const float* dbf, const float* w, const float* b, const float* gamma,
+                          int rows, int cols, float* dw, float* db, float* dgamma, void* stream);
+
 #ifdef __cplusplus
 }
 #endif

@@ -118,6 +118,6 @@ EXPORTED_SYMBOLS = (
     "m3l_attention_long_fwd", "m3l_attention_long_bwd",
     "m3l_attention_dh_fwd", "m3l_attention_dh_bwd", "m3l_attention_dropout_fwd", "m3l_attention_dropout_bwd",
     "m3l_dropout_bwd", "m3l_grad_sumsq", "m3l_optimizer_step_begin", "m3l_clip_adamw", "m3l_cast_bf16",
-    "m3l_transpose_cast_bf16", "m3l_token_mean_fwd", "m3l_token_mean_bwd",
+    "m3l_transpose_cast_bf16", "m3l_layerscale_fold", "m3l_layerscale_unfold", "m3l_token_mean_fwd", "m3l_token_mean_bwd",
     "m3l_im2col", "m3l_col2im_relu", "m3l_token_finish", "m3l_token_finish_bwd", "m3l_vt_load", "m3l_patchify", "m3l_row_scatter_add", "m3l_ema_update",
 )

@@ -630,6 +630,33 @@ def transpose_cast_bf16(src_base, dst_base, descs_dev, count):
                                               current_stream()), "m3l_transpose_cast_bf16")
 
 
+def layerscale_fold(w, b, gamma, wf, wf_t=None, bf=None):
+    """wf = bf16(gamma[:, None] * w) (gamma None: bf16(w)), wf_t = its transpose, bf = gamma * b, all in place
+    (w fp32 [rows, cols]; rounded exactly as torch rounds the same expression)."""
+    _req_cuda(w, b, gamma, wf, wf_t, bf)
+    rows, cols = w.shape
+    assert w.dtype == torch.float32 and w.is_contiguous()
+    assert wf.dtype == torch.bfloat16 and wf.is_contiguous() and wf.shape == (rows, cols)
+    assert wf_t is None or (wf_t.dtype == torch.bfloat16 and wf_t.is_contiguous() and wf_t.shape == (cols, rows))
+    for v in (b, gamma, bf):
+        assert v is None or (v.dtype == torch.float32 and v.is_contiguous() and v.numel() == rows)
+    check(_lib.load().m3l_layerscale_fold(ptr(w), ptr(b), ptr(gamma), rows, cols, ptr(wf), ptr(wf_t), ptr(bf),
+                                          current_stream()), "m3l_layerscale_fold")
+
+
+def layerscale_unfold(dwf, dbf, w, b, gamma, dw, db, dgamma):
+    """Gradients of (w, b, gamma) from those of the folded Linear (w' = gamma o w, b' = gamma o b): dw = gamma o dwf,
+    db = gamma o dbf, dgamma = rowsum(w o dwf) + b o dbf (all fp32, written)."""
+    _req_cuda(dwf, dbf, w, b, gamma, dw, db, dgamma)
+    rows, cols = w.shape
+    for m in (dwf, w, dw):
+        assert m.dtype == torch.float32 and m.is_contiguous() and m.shape == (rows, cols)
+    for v in (dbf, b, gamma, db, dgamma):
+        assert v.dtype == torch.float32 and v.is_contiguous() and v.numel() == rows
+    check(_lib.load().m3l_layerscale_unfold(ptr(dwf), ptr(dbf), ptr(w), ptr(b), ptr(gamma), rows, cols, ptr(dw),
+                                            ptr(db), ptr(dgamma), current_stream()), "m3l_layerscale_unfold")
+
+
 # ------------------------------------------------------------------------------------------
 # launch accounting (bench.py reports how many of our kernels run per step)
 # ------------------------------------------------------------------------------------------
