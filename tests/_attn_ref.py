@@ -66,6 +66,12 @@ def _rounded(x, e):
     return torch.maximum(rb(x, e), torch.where(x.abs() < FLUSH, x.abs() + e, torch.zeros_like(x)))
 
 
+def kacc_model(m, T=0):
+    """Relative error bound of an m-term fp32 tensor-core contraction of exact bf16 x bf16 products: one rounding (or
+    truncation: 2^-23) per 16-term step, one for the first product, and one per rescale of the accumulator (T)."""
+    return (math.ceil(m / 16) + 1 + T) * 2.0 ** -23
+
+
 def split_qkv(qkv, B, n, H, dh):
     """[B*n, 3*H*dh] -> q, k, v [B, H, n, dh] (float64)."""
     q, k, v = qkv.double().view(B, n, 3, H, dh).permute(2, 0, 3, 1, 4)
@@ -104,7 +110,7 @@ def forward_reference(qkv, B, n, H, dh, scale):
     es = (dh / 16 + 3) * 2.0 ** -23 * scale * (q.abs() @ k.abs().transpose(-1, -2)).amax(-1, keepdim=True)
     smax = S.abs().amax(-1, keepdim=True)
     ef = C * (2 * es + 2.0 ** -21 * smax + 2.0 ** -22 * T)
-    kacc = lambda m_: (math.ceil(m_ / 16) + 1 + T) * 2.0 ** -23
+    kacc = lambda m_: kacc_model(m_, T)
     if long:
         Rf = (U * (1 + ef) + ef) * pt
     else:
@@ -170,7 +176,7 @@ def cell_distance(got, want):
     return torch.maximum(torch.maximum(lo - want, want - hi), torch.zeros_like(g))
 
 
-def worst_ratio(name, got, want, budget):
+def worst_ratio(name, got, want, budget, labels=("b", "h", "row", "col")):
     """Largest error / budget over every element, with where it occurs.  got, want, budget: [B, H, n(, dh)].  A bf16
     got is measured by cell_distance (the error its fp32 value must have had), an fp32 one by |got - want|.
     Returns (ratio, message); a non-finite element, or an error where the budget is zero, gives ratio inf."""
@@ -181,7 +187,6 @@ def worst_ratio(name, got, want, budget):
     ratio = torch.where(torch.isfinite(got), ratio, torch.full_like(ratio, math.inf))
     idx = int(ratio.flatten().argmax())
     where = list(torch.unravel_index(torch.tensor(idx), ratio.shape))
-    labels = ("b", "h", "row", "col")
     loc = ", ".join(f"{l}={int(i)}" for l, i in zip(labels, where))
     r = float(ratio.flatten()[idx])
     msg = (f"{name}: worst |err| / budget = {r:.3g} at ({loc}): got {float(got.flatten()[idx]):.6g}, "
